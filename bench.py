@@ -7,6 +7,8 @@
 The default workload is config 3 (adaptive DoPri5, 10^6 Van der Pol oscillators), the configuration the north-star target is
 quoted on; at N = 1 the other configs are measured in the same run and reported under `also`, each with its own roofline.
   python bench.py --impl reference ...      # the CPU restatement of the reference path on the host cores
+  python bench.py --dump-outputs DIR ...    # also write what the last timed step computed, DIR/<name>.npy: the same arguments give the
+                                            # same inputs on every run, so two builds can be compared output for output
 
 A "step" is ONE pass of the hot path over ONE batch: one kernel launch that advances every trajectory of a
 10^6-trajectory ensemble by one RK step (lorenz_rk4) / one adaptive attempt (vdp_dopri5), or one RK4 step of the
@@ -96,7 +98,37 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------------------------------
 # workloads
 # ---------------------------------------------------------------------------------------------------------------------
-class LorenzRK4:
+def solver_outputs(s, x):
+    """What a caller reads back after a solver's last step: the state `x` and, per trajectory, its time and next step size."""
+    st = s.stats()
+    return {"x": x, "t": st["t"], "h": st["h"]}
+
+
+class Batches:
+    """Independent batches of one ensemble (`solvers`, all started from `x0`), one launch each in turn (vo.step_many)."""
+    adaptive = False
+
+    def restart(self):
+        """Every batch back to its initial state, then its first call (the Chkpt event at t0, no launch), as after construction."""
+        for s in self.solvers:
+            s.reset(self.x0)
+        self.vo.step_many(self.solvers, self.adaptive, 1)
+
+    def run_steps(self, k):
+        nb = len(self.solvers)
+        if k >= nb:
+            self.vo.step_many(self.solvers, self.adaptive, k // nb)
+        if k % nb:
+            self.vo.step_many(self.solvers[: k % nb], self.adaptive, 1)
+        if k:
+            self.last = self.solvers[(k % nb or nb) - 1]
+
+    def outputs(self):
+        """The batch the last step advanced."""
+        return solver_outputs(self.last, self.last.current()[1].to_host())
+
+
+class LorenzRK4(Batches):
     name = "lorenz_rk4"
     label = "config 2: fixed-step RK4, 10^6 Lorenz-63 trajectories per batch, f64, h=1e-3"
     bytes_per_unit = 48.0  # SURVEY.md §8(d): read state + write state, 2*d*8
@@ -113,13 +145,6 @@ class LorenzRK4:
         self.x0 = vo.Ensemble.from_host(ctx, self.x0_host)
         self.solvers = [vo.RK45Solver(self.rhs, 0.0, 1.0e9, self.x0, 1e-3, tableau=self.tableau) for _ in range(n_batches)]
         vo.step_many(self.solvers, False, 1)  # the first call of every solver is the Chkpt event at t0 (no launch)
-
-    def run_steps(self, k):
-        nb = len(self.solvers)
-        if k >= nb:
-            self.vo.step_many(self.solvers, False, k // nb)
-        if k % nb:
-            self.vo.step_many(self.solvers[: k % nb], False, 1)
 
     def units(self, k):
         return float(k) * N_TRAJ
@@ -150,12 +175,13 @@ class LorenzRK4:
         return float(sum(st.counts["Step"] for st in sts)), self.pin_in.numel() * 8, self.pin_out.numel() * 8
 
 
-class VdpDopri5:
+class VdpDopri5(Batches):
     name = "vdp_dopri5"
     label = "config 3: adaptive DoPri5, 10^6 Van der Pol oscillators per batch (mu sweep 0.5..20), rtol 1e-6, per-trajectory control"
     bytes_per_unit = 80.0  # SURVEY.md §8(d): state in/out + t,h,prev_h in/out
     unit_name = "attempted trajectory-step"
     state_mb = 60
+    adaptive = True
 
     def __init__(self, vo, ctx, rank, world, n_batches):
         self.vo, self.ctx = vo, ctx
@@ -178,13 +204,6 @@ class VdpDopri5:
                 s_.set_mixed_stepping(True)
         vo.step_many(self.solvers, True, 1)
         self._attempts0 = None
-
-    def run_steps(self, k):
-        nb = len(self.solvers)
-        if k >= nb:
-            self.vo.step_many(self.solvers, True, k // nb)
-        if k % nb:
-            self.vo.step_many(self.solvers[: k % nb], True, 1)
 
     def attempts(self):
         tot = 0
@@ -246,8 +265,15 @@ class HeatRK4:
         self.solvers = [vo.RK45Solver(self.rhs, 0.0, 1.0e9, self.x0, 0.25, tableau=self.tableau)]
         self.solvers[0].step()
 
+    def restart(self):
+        self.solvers[0].reset(self.x0)
+        self.solvers[0].step()
+
     def run_steps(self, k):
         self.vo.step_many(self.solvers, False, k)
+
+    def outputs(self):
+        return solver_outputs(self.solvers[0], self.solvers[0].current()[1].to_host()[0])
 
     def units(self, k):
         return float(k) * self.D
@@ -299,10 +325,18 @@ class HeatRK4DD:
         self.ds = vo.domain.HeatSlabSolver(ctx, self.D, lambda j: vo.workloads.heat_u0_at(j, self.D), 1.0, 0.0, 1.0e9, 0.25, steps_per_exchange=DD_K)
         self.ds.step()  # Chkpt at t0
         self.solvers = []
+        self.x0 = vo.Ensemble.from_host(ctx, vo.workloads.heat_u0_at(self.ds.slab.global_index(), self.D)[None, :])  # the slab, ghosts included
+
+    def restart(self):
+        self.ds.reset(self.x0)
+        self.ds.step()
 
     def run_steps(self, k):
         for _ in range(k):
             self.ds.step()
+
+    def outputs(self):
+        return solver_outputs(self.ds.solver, self.ds.local_interior())
 
     def units(self, k):
         return float(k) * self.ds.slab.m  # owned points only: the ghost points are redundant work
@@ -421,8 +455,16 @@ class SchrodingerCFM4:
         self.flops_per_unit_bound = float(_plan_terms(bound[:: max(1, len(bound) // 4096)]).mean()) * 2 * 2 * 8 * self.NDIM ** 2
         self.bytes_per_unit = None
 
+    def restart(self):
+        self.solver.reset()  # back to the initial states the solver keeps on the device
+        self.solver.step()
+
     def run_steps(self, k):
         self.solver.run(max_calls=k)
+
+    def outputs(self):
+        st = self.solver.stats()
+        return {"psi": self.solver.current()[1].view(np.float64).reshape(self.N_SYS, self.NDIM, 2), "t": st["t"], "h": st["h"]}
 
     def units(self, k):
         return float(k) * self.N_SYS
@@ -838,6 +880,23 @@ def numa_bind(torch, local):
 # with, 2 GPUs). 0 switches it off.
 GATE_US = float(os.environ.get("VECODE_BENCH_GATE_US", "150"))
 SPIN_UP_MS = 40.0  # untimed load right before the timed region, whatever --warmup says: clocks and caches in their steady state
+DUMP_BYTES = 64_000_000  # --dump-outputs: all files together, headers included
+
+
+def dump_outputs(path, arrays):
+    """Writes `arrays` as path/<name>.npy in float64. Above DUMP_BYTES in all, the arrays of the most rows keep a fixed seeded sample of
+    their rows (the same rows for each, ascending), whose indices go to path/rows.npy."""
+    n = max(len(a) for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        per_row = sum(a.nbytes // n for a in arrays.values() if len(a) == n) + 8
+        rest = sum(a.nbytes for a in arrays.values() if len(a) != n) + 4096 * (len(arrays) + 1)
+        rows = np.sort(np.random.default_rng(0).choice(n, (DUMP_BYTES - rest) // per_row, replace=False))
+        arrays = {k: a[rows] if len(a) == n else a for k, a in arrays.items()}
+        arrays["rows"] = rows
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def main():
@@ -857,7 +916,13 @@ def main():
     ap.add_argument("--n-traj", type=int, default=N_TRAJ, help="trajectories per batch (experiments only; the named configs use 10^6)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-also", action="store_true", help="skip the secondary workload summary")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64, rank 0's "
+                    f"trajectories, at most {DUMP_BYTES // 1_000_000} MB in all: a fixed sample of the rows of a larger output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl b200)")
     args.warmup = max(args.warmup, 3)
     N_TRAJ = args.n_traj
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
@@ -914,6 +979,10 @@ def main():
             per_step_ms = max_over_ranks(per_step_ms)  # every rank runs the same number of spin-up steps (heat_rk4_dd has a collective inside)
         spin = int(min(max(SPIN_UP_MS / per_step_ms, 1), 100000))
         w2.run_steps(spin)
+        # the spin-up's length follows the measured step time: start over, so that what the warm-up and the timed steps compute depends
+        # on the arguments alone (two builds compare output for output, --dump-outputs)
+        w2.restart()
+        w2.run_steps(max(nb, 1))
         w2.run_steps(warmup)
         if sync_ranks:
             barrier()
@@ -944,6 +1013,7 @@ def main():
         sampler.start()
     t_wall0 = time.time()
     w, ctx, n_batches, ms, launches, units_per_rank = device_leg(W, args.arith, args.steps, args.warmup, args.events_per_launch, rank, world, sync_ranks=True)
+    outputs = w.outputs() if args.dump_outputs and rank == 0 else None  # before the load below steps on
     # keep the same load up until the clock sampler has seen it (short timed regions are over before the first sample)
     while time.time() - t_wall0 < 0.6:
         w.run_steps(max(args.steps // 4, 16))
@@ -1059,7 +1129,8 @@ def main():
                            if W not in (HeatRK4, HeatRK4Fused, HeatRK4DD, SchrodingerCFM4, SchrodingerMagnusDense, SchrodingerMagnusApplied) else ("state 512 MB per buffer > 126 MB L2" if W in (HeatRK4, HeatRK4Fused) else
                                                                         f"slab of {512 // world} MB per buffer per GPU" if W is HeatRK4DD else
                                                                         "compute-bound: 102 MB of state per launch, streamed once"),
-                           "warmup_note": f"every batch touched once, then ~{SPIN_UP_MS:.0f} ms of the same launches and the {args.warmup} warm-up steps, all untimed, before the {args.steps} timed steps",
+                           "warmup_note": f"every batch touched once, then ~{SPIN_UP_MS:.0f} ms of the same launches, a restart from the initial state with every batch "
+                                          f"touched once more, and the {args.warmup} warm-up steps, all untimed, before the {args.steps} timed steps",
                            "timing": ((f"barrier + synchronize, a {GATE_US:.0f} us blocking kernel (torch.cuda._sleep, untimed), event, {args.steps} steps, event, barrier + synchronize: the "
                                        "launches are queued behind the blocking kernel, so the events bracket device time of the steps (VECODE_BENCH_GATE_US=0: without). "
                                        if GATE_US > 0 else "barrier + synchronize, event, steps, event, barrier + synchronize (no blocking kernel). ") +
@@ -1081,6 +1152,8 @@ def main():
             line["cpu_baseline"] = cpu
         if also:
             line["also"] = also
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
