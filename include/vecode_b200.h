@@ -271,12 +271,10 @@ int32_t vo_solver_set_record_dx_norm(vo_solver s, int32_t on);
  * checkpoint with a prev_h that was never written, so it returns VO_ERR_STATE unless mixed stepping was switched on (1)
  * before the first adaptive step — the kernels then store prev_h on every attempt like the reference. Default 0. */
 int32_t vo_solver_set_mixed_stepping(vo_solver s, int32_t on);
-/* 1: run the one-event adaptive sweep (vo_step_adaptive / vo_step_many on ensembles of >= 1024 trajectories with an unrolled
- * stage count) on a tile-blocked private copy of the state — one contiguous block per 64 trajectories holding x, the
- * per-trajectory parameters and every controller scalar, fetched with one bulk copy per warp — which is packed on entry to
- * such a run and unpacked before anything else reads the state (vo_current, vo_solver_stats, other kernels). Same arithmetic,
- * same bits, 4 % fewer instructions; measured no faster than the public layout (the sweep moves 92-96 B per attempt and sits
- * at 85 % of the HBM copy rate either way), so the default is 0. */
+/* The solver's state has one layout, the public one (SoA ensemble + per-trajectory controller arrays). 0 selects it and does
+ * nothing else; any other value returns VO_ERR_UNSUPPORTED: the tile-blocked private copy of the state that 1 once selected for
+ * the one-event adaptive sweep was removed, having measured no faster (the sweep moves 92-96 B per attempt and sits at 85 % of
+ * the HBM copy rate on either layout). */
 int32_t vo_solver_set_blocked(vo_solver s, int32_t on);
 
 /* ODESolver::step (ode.rs:249-253) / AdaptiveODESolver::step_adaptive (ode.rs:337-341) applied to every

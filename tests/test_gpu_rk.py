@@ -663,21 +663,21 @@ def test_run_tail_launch_on_another_kernel_is_not_chained(vo, ctx, max_calls):
     assert int(out[0][1]["accepted"].sum() + out[0][1]["rejected"].sum()) == n * (2 * max_calls - 1)  # all but the Chkpt call
 
 
-@pytest.mark.parametrize("blocked", [True, False])
+@pytest.mark.parametrize("prev_h", ["lazy", "every_attempt"])
 @pytest.mark.parametrize("tab", ["DOPRI5", "RKF45_REF"])
-def test_strict_one_event_control_kernel_against_oracle(vo, ctx, oracle, tab, blocked):
-    """The kernels bench.py times for config 3 — rk_ctl2b_kernel<.., STRICT> on the tile-blocked state (blocked) and
-    rk_ctl2w_staged_kernel<.., STRICT> on the public layout, ONE event per launch, N >= 1024 — straight
-    against the oracle: same accepted / rejected counts per trajectory and the state within rtol. (The controller's powf is
-    correctly rounded here and glibc's in the oracle, which rounds differently for about one argument in a thousand, so a
-    step size may differ in its last bit now and then: states are compared to 1e-9, not bitwise.)"""
+def test_strict_one_event_control_kernel_against_oracle(vo, ctx, oracle, tab, prev_h):
+    """The kernel bench.py times for config 3 — rk_ctl2w_staged_kernel<.., STRICT>, ONE event per launch, N >= 1024, with the
+    lazy prev_h store and with mixed stepping (prev_h stored on every attempt) — straight against the oracle: same accepted /
+    rejected counts per trajectory and the state within rtol. (The controller's powf is correctly rounded here and glibc's in
+    the oracle, which rounds differently for about one argument in a thousand, so a step size may differ in its last bit now
+    and then: states are compared to 1e-9, not bitwise.)"""
     n, rtol, tf = 2048, 1e-6, 4.0
     mu = vo.workloads.vdp_mu(n)
     x0 = vo.workloads.vdp_x0(n)
     ref = oracle.rk_ensemble("VDP", mu[:, None], oracle.builtin_tableau(oracle.TABLEAU_ID[tab]), 0.0, tf, x0, 1e-3, n_threads=8, adaptive=True, rtol=rtol)
     rhs = vo.Rhs(ctx, "VDP", 2, [mu])
     s = vo.RK45Solver(rhs, 0.0, tf, vo.Ensemble.from_host(ctx, x0), 1e-3, tableau=vo.ButcherTableu.builtin(tab)).with_tolerance(rtol, rtol)
-    s.set_events_per_launch(1).set_blocked(blocked)
+    s.set_events_per_launch(1).set_mixed_stepping(prev_h == "every_attempt")
     l0 = ctx.launch_count
     st = s.run(adaptive=True)
     assert st.kind == "Done"
@@ -775,35 +775,37 @@ def test_mixed_step_and_step_adaptive(vo, ctx, oracle):
     assert np.array_equal(s.stats()["h"], h_before_last)
 
 
-@pytest.mark.parametrize("arith", ["strict", "fast"])
-@pytest.mark.parametrize("n", [1024, 2500, 40_000])
-def test_blocked_sweep_equals_public_layout_bitwise(vo, n, arith):
-    """The one-event adaptive sweep on the tile-blocked private copy of the state (rk_small_blk.cuh) against the same sweep on
-    the public layout (rk_ctl2w_staged_kernel): same arithmetic, so every bit of the state and of the controller arrays must
-    agree — through checkpoints (the slow path inside the blocked kernel), snapshots, ragged tails (n % 256 != 0: padded
-    tiles), reads in mid-run (vo_solver_stats / vo_current unpack, the next launch goes on from the tiles), a write to the
-    borrowed ensemble (the tiles are re-packed), a parameter change and a switch to the 8-event kernel and back."""
-    c = vo.Context(0, arith=arith)
+@pytest.mark.parametrize("n", [1024, 1026, 2500, 8192, 40_000, 65_538])
+def test_one_event_sweep_equals_stage_path_bitwise(vo, n):
+    """The one-event adaptive sweep of the register-resident path (rk_small2.cuh: rk_ctl2w_staged_kernel, its slow path and
+    ragged tail through ctl_lane) against the stage path in strict arithmetic (FAST's reformulated controller exists only on
+    the register path): every bit of the state, of the controller arrays and of the snapshots must agree — through
+    checkpoints, snapshots, ragged tails (n % 256 != 0), reads in mid-run, a write to the borrowed ensemble, a parameter
+    change and a switch to the 8-event kernel and back. The public state layout is the only one: set_blocked(False) is
+    accepted, set_blocked(True) refused."""
+    c = vo.Context(0, arith="strict")
     mu = vo.workloads.vdp_mu(n)
     x0 = vo.workloads.vdp_x0(n) + 1e-3 * np.sin(np.arange(2 * n)).reshape(n, 2)
     out = []
-    for blocked in (True, False):
+    for stage_path in (False, True):
         rhs = vo.Rhs(c, "VDP", 2, [mu])
         s = vo.RK45Solver(rhs, 0.0, 1.5, vo.Ensemble.from_host(c, x0), 1e-3, tableau=vo.ButcherTableu.builtin("DOPRI5")).with_tolerance(1e-6, 1e-6)
-        s.set_blocked(blocked).set_events_per_launch(1).set_t_list([0.0, 0.4, 1.0, 1.5]).enable_snapshots()
+        s.set_blocked(False).set_stage_path(stage_path).set_events_per_launch(1).set_t_list([0.0, 0.4, 1.0, 1.5]).enable_snapshots()
+        with pytest.raises(vo.VecOdeError):
+            s.set_blocked(True)
         for _ in range(25):
             s.step_adaptive()
-        mid = s.stats()                                   # unpack; both layouts valid
+        mid = s.stats()
         for _ in range(10):
             s.step_adaptive()
-        vo.LinearCombination.scale(s.current()[1], 1.0 + 2.0 ** -30)   # the caller writes the borrowed state: tiles must be re-packed
+        vo.LinearCombination.scale(s.current()[1], 1.0 + 2.0 ** -30)   # the caller writes the borrowed state
         for _ in range(10):
             s.step_adaptive()
-        rhs.set_param(0, mu * (1.0 + 2.0 ** -20))         # a parameter changes under the tiles
+        rhs.set_param(0, mu * (1.0 + 2.0 ** -20))         # a parameter changes in mid-run
         for _ in range(10):
             s.step_adaptive()
         s.set_events_per_launch(8)
-        s.run(adaptive=True, max_calls=24)                # the 8-event kernel on the public layout ...
+        s.run(adaptive=True, max_calls=24)                # the 8-event kernel on the register-resident path ...
         s.set_events_per_launch(1)
         st = s.run(adaptive=True)                         # ... and back to the one-event sweep until every trajectory is done
         assert st.kind == "Done"

@@ -529,7 +529,8 @@ class RK45Solver:
         return self
 
     def set_blocked(self, on: bool = True):
-        """Run the one-event adaptive sweep on the tile-blocked private copy of the state (default) or on the public layout."""
+        """False: keep the public state layout, the only one (no-op). True raises: the tile-blocked copy of the state was
+        removed as no faster (vo_solver_set_blocked)."""
         check(lib().vo_solver_set_blocked(self._h, 1 if on else 0), self.ctx._h)
         return self
 

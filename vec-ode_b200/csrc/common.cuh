@@ -66,7 +66,6 @@ struct vo_rhs_s {
     double shared[VO_MAX_PARAMS];      // shared value of each parameter
     double* per_traj[VO_MAX_PARAMS];   // device array or nullptr
     int64_t per_traj_n[VO_MAX_PARAMS];
-    uint64_t version = 0;              // bumped whenever a parameter changes (solvers that keep a packed copy of per-trajectory parameters re-pack)
     std::string body;                  // VO_RHS_CUSTOM: source of the RHS statements
     std::map<int, void*> modules;      // VO_RHS_CUSTOM: compiled modules keyed by (stage count, arithmetic mode)
     int radius = 0;                    // VO_RHS_CUSTOM_STENCIL: the stencil reaches `radius` grid points to each side

@@ -470,7 +470,7 @@ int32_t vo_rhs_num_params(vo_rhs r) { return r ? r->np : VO_ERR_BAD_ARG; }
 
 int32_t vo_rhs_set_param(vo_rhs r, int32_t idx, double value) {
     if (!r || idx < 0 || idx >= r->np) return vo_fail(r ? r->ctx : nullptr, VO_ERR_BAD_ARG, "vo_rhs_set_param: bad index");
-    r->shared[idx] = value, r->version++;
+    r->shared[idx] = value;
     if (r->per_traj[idx]) {
         DeviceGuard g(r->ctx->device);
         cudaStreamSynchronize(r->ctx->stream);
@@ -496,7 +496,6 @@ int32_t vo_rhs_set_param_array(vo_rhs r, int32_t idx, const double* host, int64_
     }
     VO_CUDA(c, cudaMemcpyAsync(r->per_traj[idx], host, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
     VO_CUDA(c, cudaStreamSynchronize(c->stream));
-    r->version++;
     return VO_OK;
 }
 

@@ -181,10 +181,6 @@ int32_t dispatch_exp(vo_split sp, const ExpKP& kp, double2* psi, double2* psi_ou
         VO_CHECK_LAUNCH(c);
         return VO_OK;
     }
-    {   // experiment switch (A/B runs): config 5's shape with tiles of 32 systems on 16 warps, the basis shared by both column groups
-        static const int tb = getenv("VECODE_EXP_TB") ? atoi(getenv("VECODE_EXP_TB")) : 16;
-        if (tb == 32 && sp->n == 64 && sp->M == 2) return launch_exp<64, 2, 32>(c, kp, sp->frag_dev, psi, psi_out, gp, coef_in, ca, ev, order, tile_ctr);
-    }
 #define VO_EXP_CASE(NDIM, MM) \
     if (sp->n == NDIM && sp->M == MM) return launch_exp<NDIM, MM, 16>(c, kp, sp->frag_dev, psi, psi_out, gp, coef_in, ca, ev, order, tile_ctr);
     VO_EXP_SHAPES(VO_EXP_CASE)

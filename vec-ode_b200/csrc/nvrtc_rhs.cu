@@ -132,11 +132,11 @@ std::string cu_msg(Driver* dr, CUresult e) {
 }
 
 // ---- one compiled module -----------------------------------------------------------------------------------------
-enum { K_FIXED_STAGED, K_FIXED, K_CTL_STAGED_GEN, K_CTL_STAGED_L2, K_CTL2_STAGED, K_CTL, K_FIXED2_STAGED, K_SMALL_COUNT };
+// function tables: a register-resident module's is indexed by SmallKernel (rk_small_launch.cuh), a stage-path module's by
 enum { K_STAGE, K_STAGE_TAIL, K_STAGE_COUNT };
 // stencil modules: the two plain kernels, then the TMA-staged ones indexed by (tail, number of stage-derivative rows read)
 constexpr int K_STENCIL_TMA = 2, K_FN_MAX = 2 + 2 * 8;
-static_assert(K_FN_MAX >= K_SMALL_COUNT, "CustomModule::fn too small");
+static_assert(K_FN_MAX >= SK_COUNT, "CustomModule::fn too small");
 constexpr int STAGE_MODULE = -1;  // `S` key of the stage-path module (it does not depend on the stage count)
 
 struct CustomModule {
@@ -175,14 +175,14 @@ std::vector<std::string> kernel_names(int S, bool strict, bool stage_module, boo
         return v;
     }
     if (stage_module) return {"stage_pointwise_kernel<RhsCustom, " + st + ", false>", "stage_pointwise_kernel<RhsCustom, " + st + ", true>"};
-    std::vector<std::string> v(K_SMALL_COUNT);
-    v[K_FIXED_STAGED] = "rk_fixed_staged_kernel<RhsCustom, " + ss + ", " + st + ">";
-    v[K_FIXED] = "rk_fixed_kernel<RhsCustom, " + ss + ", " + st + ">";
-    v[K_CTL_STAGED_GEN] = "rk_ctl_staged_kernel<RhsCustom, " + ss + ", " + st + ", 0>";
-    v[K_CTL_STAGED_L2] = "rk_ctl_staged_kernel<RhsCustom, " + ss + ", " + st + ", 1>";
-    v[K_CTL2_STAGED] = S > 0 ? "rk_ctl2w_staged_kernel<RhsCustom, " + ss + ", " + st + ">" : "";
-    v[K_CTL] = "rk_ctl_kernel<RhsCustom, " + ss + ", " + st + ">";
-    v[K_FIXED2_STAGED] = S > 0 ? "rk_fixed2w_staged_kernel<RhsCustom, " + ss + ", " + st + ">" : "";  // warp-autonomous staging, as for the compiled-in families
+    std::vector<std::string> v(SK_COUNT);
+    v[SK_FIXED2W] = S > 0 ? "rk_fixed2w_staged_kernel<RhsCustom, " + ss + ", " + st + ">" : "";  // unrolled stage counts only, as in launch_one
+    v[SK_FIXED_STAGED] = "rk_fixed_staged_kernel<RhsCustom, " + ss + ", " + st + ">";
+    v[SK_FIXED] = "rk_fixed_kernel<RhsCustom, " + ss + ", " + st + ">";
+    v[SK_CTL2W] = S > 0 ? "rk_ctl2w_staged_kernel<RhsCustom, " + ss + ", " + st + ">" : "";
+    v[SK_CTL_STAGED_L2] = "rk_ctl_staged_kernel<RhsCustom, " + ss + ", " + st + ", 1>";
+    v[SK_CTL_STAGED_GEN] = "rk_ctl_staged_kernel<RhsCustom, " + ss + ", " + st + ", 0>";
+    v[SK_CTL] = "rk_ctl_kernel<RhsCustom, " + ss + ", " + st + ">";
     return v;
 }
 
@@ -319,9 +319,7 @@ int32_t custom_grid(vo_ctx c, Driver* drv, CustomModule* m, int k, int64_t N, si
         if (drv->occupancy(&bps, m->fn[k], RK_SMALL_THREADS, smem) != CUDA_SUCCESS || bps < 1) bps = 1;
         m->bps[k] = bps, m->bps_smem[k] = smem;
     }
-    const int64_t tiles = ceil_div(N, tile);
-    const int64_t iters = ceil_div(tiles, (int64_t)c->sm_count * m->bps[k]);
-    *grid = (unsigned)ceil_div(tiles, iters);
+    *grid = grid_for(ceil_div(N, tile), c->sm_count, m->bps[k]);
     return VO_OK;
 }
 
@@ -344,7 +342,7 @@ int stage_count_key(int s) { return (s == 4 || s == 6 || s == 7) ? s : 0; }  // 
 
 }  // namespace
 
-// The register-resident path for a user RHS: same kernel choice as launch_one (rk_small_launch.cuh).
+// The register-resident path for a user RHS: the kernel small_plan chooses, as launch_one (rk_small_launch.cuh) does.
 int32_t launch_small_custom(const SmallLaunch& L, vo_rhs_s* r) {
     vo_ctx c = L.ctx;
     const bool strict = c->arith == VO_ARITH_STRICT;
@@ -359,38 +357,23 @@ int32_t launch_small_custom(const SmallLaunch& L, vo_rhs_s* r) {
     RhsParams rp = *L.rp;
     CtlArrays ca = L.ca;
     EvSlot* ev = L.ev;
-    pipe::Chain ch{};
-    const int rows = r->d + per_traj_rows(rp, r->np);
-    const bool staged = small_path_is_staged(N);
+    const SmallPlan P = small_plan(N, S > 0, r->d + per_traj_rows(rp, r->np), L.cs);
     // grid, then the chain decision (same kernel and same grid as this solver's previous launch), then the launch
-    auto go = [&](int k, size_t smem, int tile, void** args) -> int32_t {
-        unsigned grid = 0;
-        int32_t rc2 = custom_grid(c, drv, m, k, N, smem, tile, &grid);
-        if (rc2 != VO_OK) return rc2;
-        ch = L.cst->next((const void*)m->fn[k], grid, staged);
-        return custom_launch(c, drv, m->fn[k], grid, RK_SMALL_THREADS, smem, ch.chained != 0, args);
-    };
+    unsigned grid = 0;
+    rc = custom_grid(c, drv, m, P.k, N, P.smem, P.tile, &grid);
+    if (rc != VO_OK) return rc;
+    pipe::Chain ch = L.cst->next((const void*)m->fn[P.k], grid, P.staged);
+    // The driver takes the number of parameters from the kernel image: the unstaged kernels (SK_FIXED, SK_CTL) have no
+    // trailing pipe::Chain and read one pointer less of the list.
+    auto go = [&](void** args) { return custom_launch(c, drv, m->fn[P.k], grid, RK_SMALL_THREADS, P.smem, ch.chained != 0, args); };
     if (L.sl) {
         StepList sl = *L.sl;
-        if (staged) {
-            void* args[] = {&x, &N, &tb, &rp, &sl, &ch};
-            if (S > 0 && N >= 4 * VO_TILE2) return go(K_FIXED2_STAGED, (size_t)VO_STAGES * rows * VO_TILE2 * sizeof(double), VO_TILE2, args);
-            return go(K_FIXED_STAGED, (size_t)VO_STAGES * rows * VO_TILE * sizeof(double), VO_TILE, args);
-        }
-        void* args[] = {&x, &N, &tb, &rp, &sl};
-        return go(K_FIXED, 0, VO_TILE, args);
+        void* args[] = {&x, &N, &tb, &rp, &sl, &ch};
+        return go(args);
     }
     CtlShared cs = *L.cs;
-    if (staged) {
-        const bool common = cs.adaptive && cs.use_err && cs.norm_kind == VO_NORM_L2;
-        void* args[] = {&x, &N, &tb, &rp, &ca, &cs, &ev, &ch};
-        if (S > 0 && common && cs.k_events == 1 && N >= 4 * VO_TILE_CTL)
-            return go(K_CTL2_STAGED, (size_t)VO_STAGES * ((rows + 2) * VO_TILE_CTL * sizeof(double) + 3 * VO_TILE_CTL * sizeof(uint32_t)), VO_TILE_CTL, args);
-        return go(common ? K_CTL_STAGED_L2 : K_CTL_STAGED_GEN, (size_t)VO_STAGES * ((rows + 2) * VO_TILE * sizeof(double) + 3 * VO_TILE * sizeof(uint32_t)),
-                  VO_TILE, args);
-    }
-    void* args[] = {&x, &N, &tb, &rp, &ca, &cs, &ev};
-    return go(K_CTL, 0, VO_TILE, args);
+    void* args[] = {&x, &N, &tb, &rp, &ca, &cs, &ev, &ch};
+    return go(args);
 }
 
 // The stage path for a user RHS (vo_rk_try_step, vo_rhs_eval, vo_solver_set_path(1)).

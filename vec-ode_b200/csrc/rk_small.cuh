@@ -513,8 +513,7 @@ __global__ void __launch_bounds__(VO_TILE) rk_fixed_staged_kernel(double* __rest
     pipe::chain_exit(ch);
 }
 
-// Where one trajectory's state and controller scalars live in global memory. SoaAcc: the public layout (SoA ensemble + CtlArrays,
-// element i of every array). rk_small_blk.cuh adds the tile-blocked layout of the one-event sweep.
+// Where one trajectory's state and controller scalars live in global memory: element i of the SoA ensemble and of every CtlArrays array.
 struct SoaAcc {
     double* x;
     int64_t N;
@@ -537,8 +536,8 @@ struct SoaAcc {
 // masked write-back. Shared by the staged kernel body and its ragged tail.
 // CFG 1 = the common adaptive configuration (step_adaptive with an error estimate and the L2 norm) resolved at compile
 // time; CFG 0 = everything decided from CtlShared at run time.
-template <class RHS, int S, bool STRICT, int CFG, class ACC>
-__device__ __forceinline__ void ctl_lane(const ACC& a, const TableauDev& tb, const CtlShared& cs,
+template <class RHS, int S, bool STRICT, int CFG>
+__device__ __forceinline__ void ctl_lane(const SoaAcc& a, const TableauDev& tb, const CtlShared& cs,
                                          const TList& tl, uint32_t word, double (&xc)[RHS::D], const double (&p)[RHS::NP], double t, double h,
                                          uint32_t n_acc, uint32_t n_rej, unsigned& c_step, unsigned& c_chkpt, unsigned& c_rej, unsigned& c_end, unsigned& c_stuck) {
     constexpr int D = RHS::D;

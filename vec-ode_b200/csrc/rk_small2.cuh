@@ -1,21 +1,10 @@
 // rk_small2.cuh — the register-resident kernels with TWO trajectories per thread (control kernel; fixed-step kernel below).
-//
-// rk_ctl_staged_kernel (rk_small.cuh) is bound by the FP64 pipe and by instruction issue, not by HBM: an adaptive
-// DoPri5 attempt of a 2-component system is one long dependent chain with ILP 2. Giving every thread two independent
-// trajectories doubles the ILP, and everything that is per-thread rather than per-trajectory — tableau coefficient
-// loads into uniform registers, loop and barrier overhead, address arithmetic shared by the pair — is paid once per two
-// attempts. Arithmetic per trajectory is unchanged (same operations, same order), so results are bit-identical to the
-// one-trajectory kernel. Tile = 256 trajectories per CTA iteration (thread t owns trajectories t and t + 128 of the tile).
-// Compiled for the common adaptive configuration (step_adaptive, error estimate present, L2 norm); everything else, and
-// the ragged tail of the ensemble, goes through ctl_lane of rk_small.cuh.
+// Arithmetic per trajectory is that of the one-trajectory kernels of rk_small.cuh (same operations, same order), so results
+// are bit-identical to them.
 #pragma once
 #include "rk_small.cuh"
 
-#define VO_TILE2 256
-#ifndef VO_CTL_U
-#define VO_CTL_U 2  // trajectories per thread of the control kernel
-#endif
-#define VO_TILE_CTL (128 * VO_CTL_U)
+#define VO_TILE2 256  // trajectories per CTA tile of both two-trajectory kernels
 
 // rk_step (rk.rs:90-155) for U independent trajectories, interleaved statement by statement.
 template <class RHS, int S, bool STRICT, int U>
@@ -61,11 +50,7 @@ __device__ __forceinline__ void rk_attempt_n(const TableauDev& tb, const double 
         for (int c = 0; c < D; ++c) xe[u][c] = A::sub(xe[u][c], xf[u][c]);  // x_err = X_b - X_berr (rk.rs:147)
 }
 
-// ---- lock-step fixed-step kernel, two trajectories per thread ------------------------------------------------------
-// rk_fixed_staged_kernel spends more issue slots on what is per THREAD (tableau coefficients into uniform registers, tile
-// addressing, barrier, loop) than on the ~70-100 FP64 operations of an RK4 step of a 3-component system, and at 10^6
-// trajectories per launch that — not HBM — sets its time (an L2-resident ensemble runs no faster). Two trajectories per
-// thread halve that overhead per trajectory and double the ILP; per-trajectory arithmetic is unchanged, so the bits are too.
+// rk_step without the error branch's difference (lock-step fixed steps) for U independent trajectories sharing t and dt.
 template <class RHS, int S, bool STRICT, int U>
 __device__ __forceinline__ void rk_attempt_fixed_n(const TableauDev& tb, bool use_err, double t, double dt, const double (&x0)[U][RHS::D],
                                                    const double (&p)[U][RHS::NP], double (&xf)[U][RHS::D]) {
@@ -102,250 +87,23 @@ __device__ __forceinline__ void rk_attempt_fixed_n(const TableauDev& tb, bool us
     }
 }
 
-template <class RHS, int S, bool STRICT>
-__global__ void __launch_bounds__(128) rk_fixed2_staged_kernel(double* __restrict__ x, int64_t N, const __grid_constant__ TableauDev tb,
-                                                               const __grid_constant__ RhsParams rp, const __grid_constant__ StepList sl,
-                                                               const pipe::Chain ch) {
-    constexpr int D = RHS::D, NP = RHS::NP, T = VO_TILE2, U = 2;
-    extern __shared__ __align__(128) double sbuf[];  // [VO_STAGES][nrows][T]
-    __shared__ __align__(8) uint64_t full[VO_STAGES];
-    int nrows = D;
-#pragma unroll
-    for (int q = 0; q < NP; ++q) nrows += rp.per_traj[q] ? 1 : 0;
-    const int64_t n_full = N / T, G = gridDim.x, first = blockIdx.x;
-    const int64_t my_count = first < n_full ? (n_full - first + G - 1) / G : 0;
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int s = 0; s < VO_STAGES; ++s) pipe::mbar_init(&full[s], 1);
-        pipe::fence_mbar_init();
-    }
-    pipe::chain_enter(ch);
-    auto issue = [&](int64_t k) {  // thread 0: all rows of this CTA's k-th tile into stage k % VO_STAGES
-        const int st = (int)(k % VO_STAGES);
-        const int64_t base = (first + k * G) * T;
-        double* dst = sbuf + (size_t)st * nrows * T;
-        pipe::mbar_expect_tx(&full[st], (uint32_t)(nrows * T * sizeof(double)));
-        int r = 0;
-#pragma unroll
-        for (int c = 0; c < D; ++c) pipe::bulk_g2s(dst + (r++) * T, x + c * N + base, T * sizeof(double), &full[st]);
-#pragma unroll
-        for (int q = 0; q < NP; ++q)
-            if (rp.per_traj[q]) pipe::bulk_g2s(dst + (r++) * T, rp.per_traj[q] + base, T * sizeof(double), &full[st]);
-    };
-    if (threadIdx.x == 0)
-        for (int64_t k = 0; k < my_count && k < VO_STAGES; ++k) issue(k);
-    for (int64_t k = 0; k < my_count; ++k) {
-        const int st = (int)(k % VO_STAGES);
-        const int64_t i0 = (first + k * G) * T + threadIdx.x;
-        pipe::mbar_wait(&full[st], (uint32_t)((k / VO_STAGES) & 1));
-        double xc[U][D], p[U][NP];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const double* src = sbuf + (size_t)st * nrows * T + threadIdx.x + 128 * u;
-            int r = 0;
-#pragma unroll
-            for (int c = 0; c < D; ++c) xc[u][c] = src[(r++) * T];
-#pragma unroll
-            for (int q = 0; q < NP; ++q) p[u][q] = rp.per_traj[q] ? src[(r++) * T] : rp.shared[q];
-        }
-        __syncthreads();  // every lane has taken its elements: the stage may be refilled
-        if (threadIdx.x == 0 && k + VO_STAGES < my_count) issue(k + VO_STAGES);
-        for (int e = 0; e < sl.n; ++e) {
-            double xf[U][D];
-            rk_attempt_fixed_n<RHS, S, STRICT, U>(tb, sl.use_err != 0, sl.t[e], sl.dt[e], xc, p, xf);
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-#pragma unroll
-                for (int c = 0; c < D; ++c) xc[u][c] = xf[u][c];
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u)
-#pragma unroll
-            for (int c = 0; c < D; ++c) x[c * N + i0 + 128 * u] = xc[u][c];
-    }
-    // ragged tail (N % 256 trajectories): plain loads, last CTA, one trajectory at a time
-    if (blockIdx.x == G - 1) {
-        for (int64_t i = n_full * T + threadIdx.x; i < N; i += 128) {
-            double xc[D], p[NP];
-            lane_load<RHS>(x, N, rp, i, xc, p);
-            for (int e = 0; e < sl.n; ++e) {
-                double xf[D], xe[D];
-                rk_attempt<RHS, S, STRICT>(tb, sl.use_err != 0, sl.t[e], sl.dt[e], xc, p, xf, xe);
-#pragma unroll
-                for (int c = 0; c < D; ++c) xc[c] = xf[c];
-            }
-#pragma unroll
-            for (int c = 0; c < D; ++c) x[c * N + i] = xc[c];
-        }
-    }
-    pipe::chain_exit(ch);
-}
-
-#ifndef VO_CTL2_MIN_BLOCKS
-#define VO_CTL2_MIN_BLOCKS 3
-#endif
-template <class RHS, int S, bool STRICT>
-__global__ void __launch_bounds__(128, VO_CTL2_MIN_BLOCKS) rk_ctl2_staged_kernel(double* __restrict__ x, int64_t N, const __grid_constant__ TableauDev tb,
-                                                                const __grid_constant__ RhsParams rp, const CtlArrays ca,
-                                                                const __grid_constant__ CtlShared cs, EvSlot* __restrict__ ev, const pipe::Chain ch) {
-    constexpr int D = RHS::D, NP = RHS::NP, T = VO_TILE_CTL, U = VO_CTL_U;
-    extern __shared__ __align__(128) double sbuf[];  // [VO_STAGES][nrows][T] doubles, then [VO_STAGES][3][T] words
-    __shared__ __align__(8) uint64_t full[VO_STAGES];
-    int nrows = D + 2;  // state, t, h
-#pragma unroll
-    for (int q = 0; q < NP; ++q) nrows += rp.per_traj[q] ? 1 : 0;
-    uint32_t* wbuf = reinterpret_cast<uint32_t*>(sbuf + (size_t)VO_STAGES * nrows * T);
-    const int64_t n_full = N / T, G = gridDim.x, first = blockIdx.x;
-    const int64_t my_count = first < n_full ? (n_full - first + G - 1) / G : 0;
-    __shared__ double s_tl[VO_INLINE_TLIST];
-    const TList tl = tlist_stage(cs, s_tl);
-    unsigned c_step = 0, c_chkpt = 0, c_rej = 0, c_end = 0, c_stuck = 0;
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int s = 0; s < VO_STAGES; ++s) pipe::mbar_init(&full[s], 1);
-        pipe::fence_mbar_init();
-    }
-    pipe::chain_enter(ch);
-    auto issue = [&](int64_t k) {
-        const int st = (int)(k % VO_STAGES);
-        const int64_t base = (first + k * G) * T;
-        double* dst = sbuf + (size_t)st * nrows * T;
-        pipe::mbar_expect_tx(&full[st], (uint32_t)(nrows * T * sizeof(double) + 3 * T * sizeof(uint32_t)));
-        int r = 0;
-#pragma unroll
-        for (int c = 0; c < D; ++c) pipe::bulk_g2s(dst + (r++) * T, x + c * N + base, T * sizeof(double), &full[st]);
-        pipe::bulk_g2s(dst + (r++) * T, ca.t + base, T * sizeof(double), &full[st]);
-        pipe::bulk_g2s(dst + (r++) * T, ca.h + base, T * sizeof(double), &full[st]);
-#pragma unroll
-        for (int q = 0; q < NP; ++q)
-            if (rp.per_traj[q]) pipe::bulk_g2s(dst + (r++) * T, rp.per_traj[q] + base, T * sizeof(double), &full[st]);
-        uint32_t* wdst = wbuf + (size_t)st * 3 * T;  // status word, accepted, rejected
-        pipe::bulk_g2s(wdst, ca.word + base, T * sizeof(uint32_t), &full[st]);
-        pipe::bulk_g2s(wdst + T, ca.n_accept + base, T * sizeof(uint32_t), &full[st]);
-        pipe::bulk_g2s(wdst + 2 * T, ca.n_reject + base, T * sizeof(uint32_t), &full[st]);
-    };
-    if (threadIdx.x == 0)
-        for (int64_t k = 0; k < my_count && k < VO_STAGES; ++k) issue(k);
-    for (int64_t k = 0; k < my_count; ++k) {
-        const int st = (int)(k % VO_STAGES);
-        const int64_t base = (first + k * G) * T;
-        pipe::mbar_wait(&full[st], (uint32_t)((k / VO_STAGES) & 1));
-        double xc[U][D], p[U][NP], t[U], h[U];
-        uint32_t word[U], n_acc[U], n_rej[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const double* src = sbuf + (size_t)st * nrows * T + threadIdx.x + 128 * u;
-            int r = 0;
-#pragma unroll
-            for (int c = 0; c < D; ++c) xc[u][c] = src[(r++) * T];
-            t[u] = src[(r++) * T], h[u] = src[(r++) * T];
-#pragma unroll
-            for (int q = 0; q < NP; ++q) p[u][q] = rp.per_traj[q] ? src[(r++) * T] : rp.shared[q];
-            const uint32_t* wsrc = wbuf + (size_t)st * 3 * T + threadIdx.x + 128 * u;
-            word[u] = wsrc[0], n_acc[u] = wsrc[T], n_rej[u] = wsrc[2 * T];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0 && k + VO_STAGES < my_count) issue(k + VO_STAGES);
-        bool live[U];
-        // fast path: one event per launch and all of the thread's trajectories take a Step (the steady state of an adaptive sweep)
-        bool pair = cs.k_events == 1;
-#pragma unroll
-        for (int u = 0; u < U; ++u) live[u] = !((word[u] >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE), pair = pair && live[u];
-        double dt[U], t_tgt[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) dt[u] = 0.0, t_tgt[u] = 0.0;
-        if (pair) {
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-                const int tgt = (int)(word[u] & VO_WORD_TGT_MASK);
-                if (tgt >= cs.n_tlist) {
-                    pair = false;
-                } else {
-                    t_tgt[u] = tl.at(tgt);
-                    const double rem = t_tgt[u] - t[u];  // step_size_of (ode.rs:165-176) + check_step (ode.rs:389-399)
-                    if (fabs(rem) <= 2.220446049250313e-16) pair = false;
-                    dt[u] = rem < h[u] ? rem : h[u];
-                }
-            }
-        }
-        if (pair) {
-            double xf[U][D], xe[U][D];
-            rk_attempt_n<RHS, S, STRICT, U>(tb, t, dt, xc, p, xf, xe);
-            double dxn[U], new_h[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) dxn[u] = 0.0;
-            bool rej[U], nonfin[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u) {  // handle_step_adaptive, ode.rs:311-334
-#ifdef VO_DIAG_NO_CTL  // diagnostic build only (tools/build_variant.sh): what the controller arithmetic costs
-                dxn[u] = xe[u][0], new_h[u] = h[u], rej[u] = xe[u][1] > 1.0e30, nonfin[u] = false;
-                continue;
-#endif
-                controller_l2<STRICT>(err_sumsq<STRICT, D>(xe[u]), h[u], cs, cs.record_dx_norm != 0, dxn[u], new_h[u], rej[u], nonfin[u]);
-            }
-#pragma unroll
-            for (int u = 0; u < U; ++u) {  // apply_step (ode.rs:402-428) + masked write-back
-                const int64_t i = base + threadIdx.x + 128 * u;
-                uint32_t status = word[u] >> VO_WORD_STATUS_SHIFT;
-                if (nonfin[u]) status |= VO_TRAJ_NONFINITE;
-                if (rej[u]) {
-                    if (h[u] <= cs.min_dt) status |= VO_TRAJ_STUCK, ++c_stuck;
-                    ca.n_reject[i] = n_rej[u] + 1, ++c_rej;
-                } else {
-#pragma unroll
-                    for (int c = 0; c < D; ++c) x[c * N + i] = xf[u][c];
-                    const double t_new = t[u] + dt[u];  // advance, ode.rs:184-188
-                    ca.t[i] = t_new;
-                    ca.n_accept[i] = n_acc[u] + 1, ++c_step;
-                    // update_step_size (ode.rs:202-205) sets prev_h = h, and the only reader of prev_h is the Chkpt / End
-                    // branch (checkpoint_update, ode.rs:192-195). This trajectory's next event is one of those iff the test
-                    // of ode.rs:391 holds at t_new — evaluated here exactly as the next call will — so prev_h only has to
-                    // reach memory then: 8 bytes per attempt less on the HBM-bound sweep. (A rejected attempt leaves t where
-                    // this Step event found it, so its next event is a Step again.)
-                    if (cs.lazy_prev_h && fabs(t_tgt[u] - t_new) <= 2.220446049250313e-16) ca.prev_h[i] = h[u];
-                }
-                if (!cs.lazy_prev_h) ca.prev_h[i] = h[u];  // update_step_size on every adaptive attempt, ode.rs:202-205
-                ca.h[i] = new_h[u];
-                if (cs.record_dx_norm) ca.dx_norm[i] = dxn[u];
-                const uint32_t nw = (word[u] & VO_WORD_TGT_MASK) | (status << VO_WORD_STATUS_SHIFT);
-                if (nw != word[u]) ca.word[i] = nw;
-            }
-        } else {
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (live[u])
-                    ctl_lane<RHS, S, STRICT, 1>(SoaAcc{x, N, ca, base + threadIdx.x + 128 * u}, tb, cs, tl, word[u], xc[u], p[u], t[u], h[u], n_acc[u], n_rej[u], c_step,
-                                                c_chkpt, c_rej, c_end, c_stuck);
-        }
-    }
-    // ragged tail (N % tile trajectories): plain loads, last CTA, one trajectory at a time
-    if (blockIdx.x == G - 1) {
-        for (int64_t i = n_full * T + threadIdx.x; i < N; i += 128) {
-            const uint32_t word = ca.word[i];
-            if (!((word >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE)) {
-                double xc[D], p[NP];
-                lane_load<RHS>(x, N, rp, i, xc, p);
-                ctl_lane<RHS, S, STRICT, 1>(SoaAcc{x, N, ca, i}, tb, cs, tl, word, xc, p, ca.t[i], ca.h[i], ca.n_accept[i], ca.n_reject[i], c_step, c_chkpt, c_rej, c_end,
-                                            c_stuck);
-            }
-        }
-    }
-    ctl_count_events(cs, ev, c_step, c_chkpt, c_rej, c_end, c_stuck);
-    pipe::chain_exit(ch);
-}
-
-// ---- control kernel, warp-autonomous staging ---------------------------------------------------------------------------
-// Same arithmetic and the same tile -> CTA map as rk_ctl2_staged_kernel, but every WARP stages its own 64 trajectories of
-// the CTA tile (lane l owns trajectories 2l and 2l+1 of them): the rows arrive through a cp.async pipeline per warp
-// (16 bytes per lane per row), so there is no elected thread, no mbarrier and no __syncthreads() in the tile loop; a lane
-// reads its two trajectories with ONE 128-bit shared load per row and writes them back with 128-bit stores when both of
-// its trajectories commit the same way.
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
 
+// ---- control kernel, two trajectories per thread, warp-autonomous staging -----------------------------------------------
+// rk_ctl_staged_kernel (rk_small.cuh) is bound by the FP64 pipe and by instruction issue, not by HBM: an adaptive
+// DoPri5 attempt of a 2-component system is one long dependent chain with ILP 2. Giving every thread two independent
+// trajectories doubles the ILP, and everything that is per-thread rather than per-trajectory — tableau coefficient
+// loads into uniform registers, loop overhead, address arithmetic shared by the pair — is paid once per two attempts.
+// Tile = VO_TILE2 trajectories per CTA iteration; every WARP stages its own 64 of them (lane l owns trajectories 2l and
+// 2l+1): the rows arrive through a cp.async pipeline per warp (16 bytes per lane per row), so there is no elected thread,
+// no mbarrier and no __syncthreads() in the tile loop; a lane reads its two trajectories with ONE 128-bit shared load per
+// row and writes them back with 128-bit stores when both of its trajectories commit the same way.
+// Compiled for the common adaptive configuration (step_adaptive, error estimate present, L2 norm, one event per launch);
+// a thread whose pair does not both take a Step, and the ragged tail of the ensemble, go through ctl_lane of rk_small.cuh.
 template <class RHS, int S, bool STRICT>
-__global__ void __launch_bounds__(128, VO_CTL2_MIN_BLOCKS + 1) rk_ctl2w_staged_kernel(double* __restrict__ x, int64_t N, const __grid_constant__ TableauDev tb,
+__global__ void __launch_bounds__(128, 4) rk_ctl2w_staged_kernel(double* __restrict__ x, int64_t N, const __grid_constant__ TableauDev tb,
                                                                  const __grid_constant__ RhsParams rp, const CtlArrays ca,
                                                                  const __grid_constant__ CtlShared cs, EvSlot* __restrict__ ev, const pipe::Chain ch) {
     constexpr int D = RHS::D, NP = RHS::NP, T = VO_TILE2, U = 2, WT = 64, NST = VO_STAGES;
@@ -440,26 +198,8 @@ __global__ void __launch_bounds__(128, VO_CTL2_MIN_BLOCKS + 1) rk_ctl2w_staged_k
 #pragma unroll
             for (int u = 0; u < U; ++u) acc[u] = err_sumsq<STRICT, D>(xe[u]);
             controller_l2_n<STRICT, U>(acc, h, cs, cs.record_dx_norm != 0, dxn, new_h, rej, nonfin);  // handle_step_adaptive, ode.rs:311-334
-#ifdef VO_COMMIT_SELECT
-            // apply_step (ode.rs:402-428), branch-free: both trajectories always store — a rejected one stores back what it loaded
-            // (the same bits), an accepted one its new state. Whole 32-byte sectors of rejected trajectories are rare (the accept
-            // rate is ~2/3 and neighbours mix), so the masked version dirtied nearly every sector anyway, while its three-way
-            // branch (both accepted / both rejected / mixed) made most warps run all three paths one after the other.
-            {
-#pragma unroll
-                for (int c = 0; c < D; ++c)
-                    *reinterpret_cast<double2*>(x + c * N + i0) = make_double2(rej[0] ? xc[0][c] : xf[0][c], rej[1] ? xc[1][c] : xf[1][c]);
-                *reinterpret_cast<double2*>(ca.t + i0) = make_double2(rej[0] ? t[0] : t[0] + dt[0], rej[1] ? t[1] : t[1] + dt[1]);  // advance, ode.rs:184-188
-                *reinterpret_cast<uint2*>(ca.n_accept + i0) = make_uint2(n_acc[0] + (rej[0] ? 0u : 1u), n_acc[1] + (rej[1] ? 0u : 1u));
-                *reinterpret_cast<uint2*>(ca.n_reject + i0) = make_uint2(n_rej[0] + (rej[0] ? 1u : 0u), n_rej[1] + (rej[1] ? 1u : 0u));
-                const unsigned nr = (rej[0] ? 1u : 0u) + (rej[1] ? 1u : 0u);
-                c_rej += nr, c_step += 2u - nr;
-            }
-            if (false) {
-#else
             // apply_step (ode.rs:402-428) + masked write-back: 128-bit stores where both trajectories commit the same way
             if (!rej[0] && !rej[1]) {
-#endif
 #pragma unroll
                 for (int c = 0; c < D; ++c) *reinterpret_cast<double2*>(x + c * N + i0) = make_double2(xf[0][c], xf[1][c]);
                 *reinterpret_cast<double2*>(ca.t + i0) = make_double2(t[0] + dt[0], t[1] + dt[1]);  // advance, ode.rs:184-188
@@ -519,7 +259,11 @@ __global__ void __launch_bounds__(128, VO_CTL2_MIN_BLOCKS + 1) rk_ctl2w_staged_k
     pipe::chain_exit(ch);
 }
 
-// ---- lock-step fixed-step kernel, warp-autonomous staging (same scheme as rk_ctl2w_staged_kernel) -----------------------
+// ---- lock-step fixed-step kernel, two trajectories per thread, warp-autonomous staging (as rk_ctl2w_staged_kernel) -------
+// rk_fixed_staged_kernel spends more issue slots on what is per THREAD (tableau coefficients into uniform registers, tile
+// addressing, barrier, loop) than on the ~70-100 FP64 operations of an RK4 step of a 3-component system, and at 10^6
+// trajectories per launch that — not HBM — sets its time (an L2-resident ensemble runs no faster). Two trajectories per
+// thread halve that overhead per trajectory and double the ILP.
 template <class RHS, int S, bool STRICT>
 __global__ void __launch_bounds__(128) rk_fixed2w_staged_kernel(double* __restrict__ x, int64_t N, const __grid_constant__ TableauDev tb,
                                                                 const __grid_constant__ RhsParams rp, const __grid_constant__ StepList sl,

@@ -6,7 +6,7 @@
 #include <tuple>
 #include <utility>
 
-#include "rk_small_blk.cuh"
+#include "rk_small2.cuh"
 
 constexpr int RK_SMALL_THREADS = 128;
 
@@ -38,16 +38,50 @@ struct SmallLaunch {
     const StepList* sl;    // lock-step fixed steps (cs == nullptr)
     EvSlot* ev;
     ChainState* cst;       // chaining state of the owning solver
-    const BlkView* blk = nullptr;  // non-NULL: the state lives in the tile-blocked copy (rk_small_blk.cuh) and x / ca are stale
 };
 
 // The staged kernels need 16-byte aligned SoA rows (N even) and at least one full tile.
 static inline bool small_path_is_staged(int64_t N) { return (N % 2 == 0) && N >= RK_SMALL_THREADS; }
 
-// Persistent grid: every CTA gets the same number of 128-trajectory tiles (no partial last wave), all CTAs resident.
+// The register-resident kernels. The order is that of a run-time compiled module's function table (nvrtc_rhs.cu).
+enum SmallKernel { SK_FIXED2W, SK_FIXED_STAGED, SK_FIXED, SK_CTL2W, SK_CTL_STAGED_L2, SK_CTL_STAGED_GEN, SK_CTL, SK_COUNT };
+
+struct SmallPlan {
+    SmallKernel k;
+    int tile;     // trajectories per CTA tile, the unit of the persistent grid
+    size_t smem;  // dynamic shared memory
+    bool staged;  // a staged kernel: chained launches (pipe::Chain)
+};
+
+// The one kernel choice of the register-resident path, for the compiled-in families (launch_one) and for run-time compiled
+// modules (launch_small_custom). `unrolled`: the stage count has a fully unrolled instantiation (S > 0); `rows`: state
+// components + per-trajectory parameter rows; `cs`: per-trajectory control, nullptr for lock-step fixed steps. The
+// two-trajectory kernels (rk_small2.cuh) need an unrolled stage count and at least four of their tiles; the control one
+// only serves the common adaptive configuration with one event per launch.
+static inline SmallPlan small_plan(int64_t N, bool unrolled, int rows, const CtlShared* cs) {
+    if (!small_path_is_staged(N)) return {cs ? SK_CTL : SK_FIXED, RK_SMALL_THREADS, 0, false};
+    const bool two = unrolled && N >= 4 * VO_TILE2;
+    if (!cs) {
+        const int tile = two ? VO_TILE2 : VO_TILE;
+        return {two ? SK_FIXED2W : SK_FIXED_STAGED, tile, (size_t)VO_STAGES * rows * tile * sizeof(double), true};
+    }
+    const bool common = cs->adaptive && cs->use_err && cs->norm_kind == VO_NORM_L2;
+    const bool ctl2 = two && common && cs->k_events == 1;
+    const int tile = ctl2 ? VO_TILE2 : VO_TILE;
+    // [stage][rows + t, h][tile] doubles, then [stage][status word, accepted, rejected][tile] words
+    const size_t smem = (size_t)VO_STAGES * ((rows + 2) * tile * sizeof(double) + 3 * tile * sizeof(uint32_t));
+    return {ctl2 ? SK_CTL2W : common ? SK_CTL_STAGED_L2 : SK_CTL_STAGED_GEN, tile, smem, true};
+}
+
+// Persistent grid: every CTA gets the same number of tiles (no partial last wave), all CTAs resident.
+static inline unsigned grid_for(int64_t tiles, int sm_count, int blocks_per_sm) {
+    const int64_t iters = ceil_div(tiles, (int64_t)sm_count * blocks_per_sm);
+    return (unsigned)ceil_div(tiles, iters);
+}
+
 // The shared-memory size depends on run-time facts (how many RHS parameters are per-trajectory arrays), and both the large
 // shared-memory opt-in and the occupancy are per device, so resident CTAs per SM are cached per (device, kernel, smem).
-template <class K> static unsigned persistent_grid(vo_ctx c, K kernel, int64_t N, size_t smem, int tile = RK_SMALL_THREADS) {
+template <class K> static unsigned persistent_grid(vo_ctx c, K kernel, int64_t N, size_t smem, int tile) {
     static std::map<std::tuple<int, const void*, size_t>, int> cache;
     static std::mutex mu;  // contexts may be driven from different host threads
     int bps;
@@ -60,9 +94,7 @@ template <class K> static unsigned persistent_grid(vo_ctx c, K kernel, int64_t N
         }
         bps = slot;
     }
-    const int64_t tiles = ceil_div(N, tile);
-    const int64_t iters = ceil_div(tiles, (int64_t)c->sm_count * bps);
-    return (unsigned)ceil_div(tiles, iters);
+    return grid_for(ceil_div(N, tile), c->sm_count, bps);
 }
 
 // A CHAINED launch (see pipe::Chain) is submitted with programmatic stream serialisation, so its CTAs are scheduled as
@@ -81,13 +113,6 @@ static void launch_staged(ChainState* cst, void (*kernel)(KArgs...), unsigned gr
     cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)..., ch);
 }
 
-// When the one-event adaptive sweep may run on the tile-blocked copy of the state: the dispatch condition of the
-// two-trajectory control kernels (below) for a compiled-in RHS family with an unrolled stage count.
-static inline bool small_path_blocked_ok(int64_t N, int stages, const CtlShared& cs) {
-    const bool unrolled = stages == 4 || stages == 6 || stages == 7;
-    return unrolled && small_path_is_staged(N) && N >= 4 * VO_TILE_CTL && cs.adaptive && cs.use_err && cs.norm_kind == VO_NORM_L2 && cs.k_events == 1;
-}
-
 static inline int per_traj_rows(const RhsParams& rp, int np) {
     int n = 0;
     for (int q = 0; q < np; ++q) n += rp.per_traj[q] ? 1 : 0;
@@ -95,60 +120,27 @@ static inline int per_traj_rows(const RhsParams& rp, int np) {
 }
 
 template <class RHS, int S, bool STRICT> static void launch_one(const SmallLaunch& L) {
-    const bool staged = small_path_is_staged(L.N);
-    if (L.sl) {
-        if (staged) {
-            if constexpr (S > 0) {
-                if (L.N >= 4 * VO_TILE2) {  // two trajectories per thread (rk_small2.cuh)
-                    const size_t smem2 = (size_t)VO_STAGES * (RHS::D + per_traj_rows(*L.rp, RHS::NP)) * VO_TILE2 * sizeof(double);
-#ifdef VO_FIXED2_CTA  // A/B switch (tools/build_variant.sh): the CTA-staged version of the kernel
-                    auto k2 = rk_fixed2_staged_kernel<RHS, S, STRICT>;
-#else
-                    auto k2 = rk_fixed2w_staged_kernel<RHS, S, STRICT>;
-#endif
-                    launch_staged(L.cst, k2, persistent_grid(L.ctx, k2, L.N, smem2, VO_TILE2), smem2, L.ctx->stream, L.x, L.N, *L.tb, *L.rp, *L.sl);
-                    return;
-                }
-            }
-            const size_t smem = (size_t)VO_STAGES * (RHS::D + per_traj_rows(*L.rp, RHS::NP)) * VO_TILE * sizeof(double);
-            auto k = rk_fixed_staged_kernel<RHS, S, STRICT>;
-            launch_staged(L.cst, k, persistent_grid(L.ctx, k, L.N, smem), smem, L.ctx->stream, L.x, L.N, *L.tb, *L.rp, *L.sl);
-        } else {
-            auto k = rk_fixed_kernel<RHS, S, STRICT>;
-            L.cst->live = false;
-            k<<<persistent_grid(L.ctx, k, L.N, 0), RK_SMALL_THREADS, 0, L.ctx->stream>>>(L.x, L.N, *L.tb, *L.rp, *L.sl);
-        }
-    } else {
-        if (staged) {
-            const size_t smem = (size_t)VO_STAGES * ((RHS::D + 2 + per_traj_rows(*L.rp, RHS::NP)) * VO_TILE * sizeof(double) + 3 * VO_TILE * sizeof(uint32_t));
-            const bool common = L.cs->adaptive && L.cs->use_err && L.cs->norm_kind == VO_NORM_L2;
-            if constexpr (S > 0) {
-                if (L.blk) {  // the one-event sweep on the tile-blocked state (solver.cu decided with small_path_blocked_ok)
-                    const size_t smemb = (size_t)4 * VO_BLK_NST * L.blk->read_bytes;
-                    auto kb = rk_ctl2b_kernel<RHS, S, STRICT>;
-                    launch_staged(L.cst, kb, persistent_grid(L.ctx, kb, L.blk->n_wtiles * VO_BLK_WT, smemb, VO_TILE_CTL), smemb, L.ctx->stream, *L.blk, L.N, *L.tb, *L.rp,
-                                  *L.cs, L.ev);
-                    return;
-                }
-                if (common && L.cs->k_events == 1 && L.N >= 4 * VO_TILE_CTL) {  // several trajectories per thread (rk_small2.cuh)
-                    const size_t smem2 = (size_t)VO_STAGES * ((RHS::D + 2 + per_traj_rows(*L.rp, RHS::NP)) * VO_TILE_CTL * sizeof(double) + 3 * VO_TILE_CTL * sizeof(uint32_t));
-#ifdef VO_CTL2_CTA  // A/B switch (tools/build_variant.sh): the CTA-staged version of the kernel
-                    auto k2 = rk_ctl2_staged_kernel<RHS, S, STRICT>;
-#else
-                    auto k2 = rk_ctl2w_staged_kernel<RHS, S, STRICT>;  // warp-autonomous staging: 15.9 against 16.9 us on the VdP sweep
-#endif
-                    launch_staged(L.cst, k2, persistent_grid(L.ctx, k2, L.N, smem2, VO_TILE_CTL), smem2, L.ctx->stream, L.x, L.N, *L.tb, *L.rp, L.ca,
-                                  *L.cs, L.ev);
-                    return;
-                }
-            }
-            auto k = common ? rk_ctl_staged_kernel<RHS, S, STRICT, 1> : rk_ctl_staged_kernel<RHS, S, STRICT, 0>;
-            launch_staged(L.cst, k, persistent_grid(L.ctx, k, L.N, smem), smem, L.ctx->stream, L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev);
-        } else {
-            auto k = rk_ctl_kernel<RHS, S, STRICT>;
-            L.cst->live = false;
-            k<<<persistent_grid(L.ctx, k, L.N, 0), RK_SMALL_THREADS, 0, L.ctx->stream>>>(L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev);
-        }
+    const SmallPlan P = small_plan(L.N, S > 0, RHS::D + per_traj_rows(*L.rp, RHS::NP), L.cs);
+    auto staged = [&](auto kernel, auto&&... args) {
+        launch_staged(L.cst, kernel, persistent_grid(L.ctx, kernel, L.N, P.smem, P.tile), P.smem, L.ctx->stream, args...);
+    };
+    auto plain = [&](auto kernel, auto&&... args) {
+        L.cst->live = false;
+        kernel<<<persistent_grid(L.ctx, kernel, L.N, 0, P.tile), RK_SMALL_THREADS, 0, L.ctx->stream>>>(args...);
+    };
+    switch (P.k) {
+        case SK_FIXED2W:
+            if constexpr (S > 0) staged(rk_fixed2w_staged_kernel<RHS, S, STRICT>, L.x, L.N, *L.tb, *L.rp, *L.sl);
+            break;
+        case SK_FIXED_STAGED: staged(rk_fixed_staged_kernel<RHS, S, STRICT>, L.x, L.N, *L.tb, *L.rp, *L.sl); break;
+        case SK_FIXED: plain(rk_fixed_kernel<RHS, S, STRICT>, L.x, L.N, *L.tb, *L.rp, *L.sl); break;
+        case SK_CTL2W:
+            if constexpr (S > 0) staged(rk_ctl2w_staged_kernel<RHS, S, STRICT>, L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev);
+            break;
+        case SK_CTL_STAGED_L2: staged(rk_ctl_staged_kernel<RHS, S, STRICT, 1>, L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev); break;
+        case SK_CTL_STAGED_GEN: staged(rk_ctl_staged_kernel<RHS, S, STRICT, 0>, L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev); break;
+        case SK_CTL: plain(rk_ctl_kernel<RHS, S, STRICT>, L.x, L.N, *L.tb, *L.rp, L.ca, *L.cs, L.ev); break;
+        case SK_COUNT: break;
     }
 }
 

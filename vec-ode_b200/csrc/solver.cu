@@ -84,14 +84,6 @@ struct vo_solver_s {
     // or of other solvers, which touch only their own state) has been enqueued on the ctx since.
     ChainState cst;
     uint64_t chain_epoch = 0;
-    // Tile-blocked copy of (x, per-trajectory parameters, controller arrays) for the one-event adaptive sweep
-    // (rk_small_blk.cuh). Exactly one of the two layouts may be stale at any time: the blocked kernel leaves the public one
-    // (x, ca) stale, every other writer leaves the tiles stale; readers call ensure_soa first.
-    BlkView bv{};
-    bool blk_valid = false, soa_valid = true;
-    uint64_t blk_par_version = 0;  // rhs->version the tiles' parameter rows were packed from
-    uint64_t both_epoch = 0;       // ctx epoch when both layouts were last known equal (a library call on the ctx since then may have written x)
-    int use_blocked = 0;           // vo_solver_set_blocked: 1 runs the one-event sweep on the tile-blocked copy (measured: no faster, see rk_small_blk.cuh)
 };
 
 namespace {
@@ -319,59 +311,6 @@ __global__ void ctl_stats_finish_kernel(unsigned long long* sums, double* mm, un
     }
 }
 
-// ---- tile-blocked copy of the state (rk_small_blk.cuh) -------------------------------------------------------------------
-BlkPackArgs blk_args(const vo_solver_s* s) {
-    BlkPackArgs a;
-    std::memset(&a, 0, sizeof a);
-    a.x = s->x->p, a.N = s->n, a.ca = s->ca, a.D = (int)s->d;
-    for (int q = 0; q < s->rhs->np; ++q)
-        if (s->rhs->per_traj[q]) a.par[a.npt++] = s->rhs->per_traj[q];
-    return a;
-}
-
-// public layout -> tiles, if the tiles are stale
-int32_t ensure_blk(vo_solver_s* s) {
-    vo_ctx c = s->ctx;
-    if (s->blk_valid && s->soa_valid && s->both_epoch != c->epoch) s->blk_valid = false;  // something on the ctx may have written x since
-    if (s->blk_valid && s->blk_par_version != s->rhs->version) {                           // a parameter changed under the tiles
-        if (!s->soa_valid) {
-            const BlkPackArgs a = blk_args(s);
-            blk_unpack_kernel<<<(unsigned)ceil_div(s->n, 256), 256, 0, c->stream>>>(s->bv, a, s->x->p);
-            VO_CHECK_LAUNCH(c);
-            s->soa_valid = true;
-        }
-        s->blk_valid = false;
-    }
-    if (s->blk_valid) return VO_OK;
-    const BlkPackArgs a = blk_args(s);
-    const int R = (int)s->d + 2 + a.npt;
-    const int64_t n_wtiles = ceil_div(s->n, VO_TILE_CTL) * (VO_TILE_CTL / VO_BLK_WT);
-    if (!s->bv.base || s->bv.R != R || s->bv.n_wtiles != n_wtiles) {
-        VO_CUDA(c, cudaStreamSynchronize(c->stream));
-        vo_dfree(s->bv.base), s->bv = BlkView{};
-        const uint32_t rb = blk_read_bytes(R);
-        if (vo_dmalloc(&s->bv.base, (size_t)n_wtiles * (rb + 1024u)) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "solver: tile-blocked state allocation failed");
-        s->bv.n_wtiles = n_wtiles, s->bv.read_bytes = rb, s->bv.stride = rb + 1024u, s->bv.R = R;
-    }
-    blk_pack_kernel<<<(unsigned)ceil_div(n_wtiles * VO_BLK_WT, 256), 256, 0, c->stream>>>(s->bv, a);
-    VO_CHECK_LAUNCH(c);
-    s->blk_valid = true, s->blk_par_version = s->rhs->version, s->both_epoch = c->epoch;
-    return VO_OK;
-}
-
-// tiles -> public layout, if the public layout is stale. `writing`: the caller is about to change x / ca, so the tiles go stale.
-int32_t ensure_soa(vo_solver_s* s, bool writing) {
-    vo_ctx c = s->ctx;
-    if (!s->soa_valid) {
-        const BlkPackArgs a = blk_args(s);
-        blk_unpack_kernel<<<(unsigned)ceil_div(s->n, 256), 256, 0, c->stream>>>(s->bv, a, s->x->p);
-        VO_CHECK_LAUNCH(c);
-        s->soa_valid = true, s->both_epoch = c->epoch;
-    }
-    if (writing) s->blk_valid = false;
-    return VO_OK;
-}
-
 // lock-step -> per-trajectory: every trajectory inherits the shared scalars.
 int32_t materialize(vo_solver_s* s) {
     if (!s->uniform) return VO_OK;
@@ -384,7 +323,7 @@ int32_t materialize(vo_solver_s* s) {
                                                                          (uint32_t)s->u_reject, word);
     VO_CHECK_LAUNCH(c);
     s->n_done = s->u_done ? s->n : 0;
-    s->uniform = false, s->blk_valid = false, s->soa_valid = true;
+    s->uniform = false;
     return VO_OK;
 }
 
@@ -421,18 +360,8 @@ int32_t launch_small(vo_solver_s* s, const CtlShared* cs, const StepList* sl) {
     vo_ctx c = s->ctx;
     const TableauDev tb = make_tableau_dev(s->tab);
     const RhsParams rp = make_rhs_params(s->rhs);
-    // the one-event adaptive sweep of a compiled-in family runs on the tile-blocked copy of the state; everything else on the public layout
-    const bool blocked = cs && !s->uniform && s->use_blocked && s->rhs->kind != VO_RHS_CUSTOM && !s->norm_rhs && small_path_blocked_ok(s->n, s->tab.s, *cs);
-    if (blocked) {
-        int32_t br = ensure_blk(s);
-        if (br != VO_OK) return br;
-        s->soa_valid = false;
-    } else if (!s->uniform) {
-        int32_t br = ensure_soa(s, true);
-        if (br != VO_OK) return br;
-    }
     if (s->chain_epoch != c->epoch) s->cst.live = false;  // something else was enqueued on the ctx since our last launch
-    SmallLaunch L{c, s->x->p, s->n, &tb, &rp, s->ca, cs, sl, s->ev_dev, &s->cst, blocked ? &s->bv : nullptr};
+    SmallLaunch L{c, s->x->p, s->n, &tb, &rp, s->ca, cs, sl, s->ev_dev, &s->cst};
     int32_t r = VO_ERR_UNSUPPORTED;
     if (s->norm_rhs) {  // a user-defined norm: the control kernels come from the run-time module that carries it
         r = launch_small_custom(L, s->norm_rhs);
@@ -747,8 +676,6 @@ int32_t stage_pertraj_event(vo_solver_s* s, bool adaptive, int* launches) {
     }
     const CtlShared cs = make_ctl_shared(s, adaptive ? 1 : 0, 1);
     const unsigned grid = (unsigned)ceil_div(s->n, 256);
-    int32_t sr = ensure_soa(s, true);
-    if (sr != VO_OK) return sr;
     ctl_prepare_kernel<<<grid, 256, 0, c->stream>>>(s->ca, cs, s->n, s->evv, s->dtv);
     VO_CHECK_LAUNCH(c);
     ++*launches;
@@ -804,10 +731,9 @@ int32_t do_events(vo_solver_s* s, bool adaptive, int k, vo_step_result* res, int
         const CtlShared cs = make_ctl_shared(s, adaptive ? 1 : 0, k);
         int32_t r = launch_small(s, &cs, nullptr);
         if (r != VO_OK) return r;
-        // the dispatch condition of the two-trajectory control kernels (launch_one, rk_small_launch.cuh), the only ones with a lazy prev_h
+        // the two-trajectory control kernel is the only one with a lazy prev_h (the plan's shared-memory size is not needed here)
         const bool unrolled = s->tab.s == 4 || s->tab.s == 6 || s->tab.s == 7;
-        if (adaptive && cs.lazy_prev_h && cs.use_err && cs.norm_kind == VO_NORM_L2 && k == 1 && unrolled && small_path_is_staged(s->n) && s->n >= 4 * VO_TILE_CTL)
-            s->prev_h_stale = true;
+        if (cs.lazy_prev_h && small_plan(s->n, unrolled, (int)s->d, &cs).k == SK_CTL2W) s->prev_h_stale = true;
         launches = 1;
         if (calls_done) *calls_done = k;
     } else {
@@ -895,7 +821,7 @@ int32_t vo_solver_destroy(vo_solver s) {
     vo_ens_destroy(s->x), vo_ens_destroy(s->next_x), vo_ens_destroy(s->x_err);
     for (vo_ens k : s->K) vo_ens_destroy(k);
     free_ctl(s);
-    vo_dfree(s->bv.base), vo_dfree(s->evv), vo_dfree(s->dtv), vo_dfree(s->norm_partial), vo_dfree(s->ev_dev), vo_dfree(s->t_list_dev), vo_dfree(s->cst.flags), vo_dfree(s->snap);
+    vo_dfree(s->evv), vo_dfree(s->dtv), vo_dfree(s->norm_partial), vo_dfree(s->ev_dev), vo_dfree(s->t_list_dev), vo_dfree(s->cst.flags), vo_dfree(s->snap);
     cudaFreeHost(s->ev_host);
     vo_dfree(s->dxn_pre);
     if (s->norm_rhs) custom_rhs_release(s->norm_rhs), delete s->norm_rhs;
@@ -990,7 +916,6 @@ int32_t vo_solver_set_h_array(vo_solver s, const double* h_host, int64_t n) {
     vo_ctx c = s->ctx;
     DeviceGuard g(c->device);
     int32_t r = materialize(s);
-    if (r == VO_OK) r = ensure_soa(s, true);
     if (r != VO_OK) return r;
     VO_CUDA(c, cudaMemcpyAsync(s->ca.h, h_host, 8 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     VO_CUDA(c, cudaMemcpyAsync(s->ca.prev_h, h_host, 8 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -1012,7 +937,7 @@ int32_t vo_solver_set_record_dx_norm(vo_solver s, int32_t on) {
 
 int32_t vo_solver_set_blocked(vo_solver s, int32_t on) {
     if (!s) return VO_ERR_BAD_ARG;
-    s->use_blocked = on ? 1 : 0;
+    if (on) return vo_fail(s->ctx, VO_ERR_UNSUPPORTED, "vo_solver_set_blocked: the tile-blocked state layout was removed (measured no faster than the public layout)");
     return VO_OK;
 }
 
@@ -1191,10 +1116,6 @@ int32_t vo_current(vo_solver s, double* t_min, double* t_max, vo_ens* x) {
     if (!s) return VO_ERR_BAD_ARG;
     vo_ctx c = s->ctx;
     DeviceGuard g(c->device);
-    if (!s->uniform) {
-        int32_t er = ensure_soa(s, false);
-        if (er != VO_OK) return er;
-    }
     if (x) *x = s->x;
     if (t_min || t_max) {
         if (s->uniform) {
@@ -1209,7 +1130,6 @@ int32_t vo_current(vo_solver s, double* t_min, double* t_max, vo_ens* x) {
             if (t_max) *t_max = *mm.second;
         }
     }
-    s->both_epoch = c->epoch;  // nothing above wrote the state; what the caller does with the borrowed ensemble moves the epoch on
     return VO_OK;
 }
 
@@ -1229,8 +1149,6 @@ int32_t vo_solver_stats(vo_solver s, int64_t* accepted, int64_t* rejected, doubl
         }
         return VO_OK;
     }
-    int32_t er = ensure_soa(s, false);
-    if (er != VO_OK) return er;
     std::vector<uint32_t> tmp(n);
     if (accepted) {
         VO_CUDA(c, cudaMemcpyAsync(tmp.data(), s->ca.n_accept, 4 * n, cudaMemcpyDeviceToHost, c->stream));
@@ -1251,7 +1169,6 @@ int32_t vo_solver_stats(vo_solver s, int64_t* accepted, int64_t* rejected, doubl
     if (h) VO_CUDA(c, cudaMemcpyAsync(h, s->ca.h, 8 * n, cudaMemcpyDeviceToHost, c->stream));
     if (dx_norm) VO_CUDA(c, cudaMemcpyAsync(dx_norm, s->ca.dx_norm, 8 * n, cudaMemcpyDeviceToHost, c->stream));
     VO_CUDA(c, cudaStreamSynchronize(c->stream));
-    s->both_epoch = c->epoch;  // read-only
     return VO_OK;
 }
 
@@ -1259,7 +1176,6 @@ int32_t vo_solver_reset(vo_solver s, vo_ens x0) {
     if (!s || !x0) return VO_ERR_BAD_ARG;
     if (x0->d != s->d || x0->n != s->n) return vo_fail(s->ctx, VO_ERR_SHAPE, "vo_solver_reset: shape mismatch");
     DeviceGuard g(s->ctx->device);
-    s->blk_valid = false, s->soa_valid = true;  // everything is overwritten
     int32_t r = vo_ens_copy(s->x, x0);
     if (r == VO_OK) r = vo_ens_copy(s->next_x, x0);
     if (r == VO_OK && s->x_err) r = vo_ens_copy(s->x_err, x0);
@@ -1288,8 +1204,6 @@ int32_t vo_solver_local_stats(vo_solver s, unsigned long long* sums_dev, double*
         VO_CUDA(c, cudaMemcpyAsync(mm_dev, h_mm, sizeof h_mm, cudaMemcpyHostToDevice, c->stream));
         return VO_OK;
     }
-    int32_t er = ensure_soa(s, false);
-    if (er != VO_OK) return er;
     const uint64_t epoch = c->epoch;
     VO_CUDA(c, cudaMemsetAsync(sums_dev, 0, 6 * sizeof(unsigned long long), c->stream));
     const long long lowest = (long long)0x8000000000000000ull;  // below the key of every double
@@ -1311,10 +1225,6 @@ int32_t vo_rk_try_step(vo_solver s, double t, double dt, vo_ens next_x, vo_ens x
     DeviceGuard g(c->device);
     if (next_x->d != s->d || next_x->n != s->n || (x_err && (x_err->d != s->d || x_err->n != s->n)))
         return vo_fail(c, VO_ERR_SHAPE, "vo_rk_try_step: shape mismatch");
-    if (!s->uniform) {
-        int32_t er = ensure_soa(s, false);
-        if (er != VO_OK) return er;
-    }
     if (K)
         for (int j = 0; j < s->tab.s; ++j)
             if (!K[j] || K[j]->d != s->d || K[j]->n != s->n) return vo_fail(c, VO_ERR_SHAPE, "vo_rk_try_step: K must hold s ensembles of the solver's shape");
