@@ -320,7 +320,9 @@ int32_t vo_rk_try_step(vo_solver s, double t, double dt, vo_ens next_x, vo_ens x
  * systems on a shared basis: an operator L_i = sum_m coef[i][m] * B_m with M complex n x n matrices B_m
  * shared by the ensemble; `L` values are coefficient ensembles, exp(L) is lazy and map_exp applies the
  * scaled Taylor series of exp(L) to the state without forming U. States: complex n-vectors, AoS
- * [N][n] interleaved (re, im). */
+ * [N][n] interleaved (re, im). n is 1 <= n <= 8 (one system per thread, FP64 in registers, a Taylor plan per system) or a
+ * multiple of 8 (the solvers run n in {16, 24, 32, 40, 48, 64} on the FP64 tensor cores, by 16-system tiles); 9 <= n <= 15 and
+ * other sizes return VO_ERR_BAD_ARG. 1 <= M <= 4. */
 int32_t vo_split_basis_create(vo_ctx ctx, int32_t n, int32_t M, const double* basis /* [M][n][n] (re,im) */,
                               vo_split* out);
 int32_t vo_split_destroy(vo_split sp);
@@ -371,8 +373,8 @@ int32_t vo_exp_destroy(vo_expsolver s);
  * `body` is CUDA C++ for statements that assign `g[1] .. g[M_gen-1]`, the real coefficients of L(t) = B_0 + sum_m g[m] B_m,
  * from `const double t` and `const double* p` (this system's 3 (M_gen - 1) parameters as handed to vo_exp_create). It is
  * compiled at run time (NVRTC, sm_100a) into the same tensor-core kernel the built-in family runs in; compile errors come
- * back through vo_last_error. vo_exp_generator_check compiles without a ctx or a GPU (n in {16, 32, 64}, M basis matrices)
- * and returns the cubin size (> 0) or a VO_ERR_* code with the compiler log in `log`. */
+ * back through vo_last_error. vo_exp_generator_check compiles without a ctx or a GPU (1 <= n <= 8, or n a multiple of 8 up to
+ * 64; M basis matrices) and returns the cubin size (> 0) or a VO_ERR_* code with the compiler log in `log`. */
 int32_t vo_exp_set_generator(vo_expsolver s, const char* body);
 /* The systems are independent, so their order on the device is free — and it matters: a tile of 16 systems runs the largest
  * Taylor degree among them. After vo_exp_set_order(s, perm, N) the solver treats device slot j as the caller's system perm[j]:
@@ -383,7 +385,8 @@ int32_t vo_exp_set_order(vo_expsolver s, const int64_t* perm, int64_t n);
  * step (one small kernel + a radix sort of N keys, ~1 % of a step of config 5) and the kernel forms its 16-system tiles in that
  * order. A tile runs the Taylor degree of its largest theta, so tiles of equal theta execute what their systems need and no more
  * (static grouping by drive amplitude cannot follow the phases). Results are those of any other order to rounding; buffers and
- * statistics stay in the caller's order. Compiled-in generator family only (a run-time compiled generator keeps the static order). */
+ * statistics stay in the caller's order. Compiled-in generator family only (a run-time compiled generator keeps the static order).
+ * For 1 <= n <= 8 every system runs its own Taylor plan and there are no tiles to group: the switch is accepted and does nothing. */
 int32_t vo_exp_set_dynamic_grouping(vo_expsolver s, int32_t on);
 int32_t vo_exp_generator_check(const char* body, int32_t n, int32_t M, char* log, int64_t log_cap);
 /* The arguments `c`, `alpha`, `alph_err` of cfm_general (exp/cfm.rs:47-52): k <= 4 nodes, alpha [rows][k] with rows <= 8

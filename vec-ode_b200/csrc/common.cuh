@@ -96,7 +96,9 @@ int32_t norm_custom_device(vo_normfn_s* f, const double* x, int64_t d, int64_t n
                            int partial_cap, bool finish);
 // a private RHS handle whose run-time modules carry the user's norm (for a compiled-in family: the family re-compiled with it)
 vo_rhs_s* custom_rhs_with_norm(const vo_rhs_s* base, const vo_normfn_s* f);
-// run-time compiled generator of the exponential integrators (nvrtc_rhs.cu): module + kernel handle for exp_step_kernel<n, M, 16, user GEN>
+// run-time compiled generator of the exponential integrators (nvrtc_rhs.cu): module + kernel handle for exp_step_kernel<n, M, 16, user GEN>,
+// or exp_small_kernel<n, M, user GEN> for n <= VO_EXP_SMALL_MAX_N
+#define VO_EXP_SMALL_MAX_N 8
 int32_t rtc_exp_module(vo_ctx c, const std::string& body, const std::string& norm_src, int ndim, int M, size_t smem, void** module_out, void** fn_out);
 int32_t rtc_exp_launch(vo_ctx c, void* fn, unsigned grid, unsigned block, size_t smem, void** args);
 void rtc_exp_unload(void* module);

@@ -14,6 +14,8 @@
 // shared operand. It runs on the FP64 tensor cores (mma.sync m8n8k4 DMMA; tcgen05 has no f64 kind): the basis lives in
 // shared memory in A-fragment order for the whole kernel, the Taylor term of the tile is re-published to shared memory
 // once per term in B-fragment-friendly layout, accumulators and the running sum stay in registers.
+// Systems of 1 <= n <= 8 levels take exp_small_kernel (exp_small_kernels.cuh) instead: one system per thread in FP64 registers,
+// the basis a kernel parameter, a Taylor plan per system, and several events per launch inside vo_exp_run.
 #include <algorithm>
 #include <cmath>
 #include <complex>
@@ -22,6 +24,18 @@
 #include <vector>
 
 #include "exp_dense_kernels.cuh"
+#include "exp_small_kernels.cuh"
+
+// Events per launch of exp_small_kernel inside vo_exp_run (a run never fuses past its readback batch of at most 16 calls). Measured
+// against one event per launch in DESIGN.md §2.3; tools/build_variant.sh rebuilds with another value for such comparisons.
+#ifndef VO_EXP_SMALL_FUSE
+#define VO_EXP_SMALL_FUSE 16
+#endif
+
+// exp_small.cu: exp_small_kernel<n, M, GenCos> for the split's shape, one thread per system
+unsigned exp_small_grid(vo_ctx c, int64_t N);
+int32_t launch_exp_small(vo_ctx c, int n, int M, const ExpKP& kp, const double* basis, double2* psi, double2* psi_out, const double* gp, const double2* coef_in,
+                         const CtlArrays& ca, EvSlot* ev);
 
 // sort_keys.cu
 size_t vo_sort_pairs_tmp_bytes(int n);
@@ -31,7 +45,8 @@ cudaError_t vo_sort_pairs(void* tmp, size_t tmp_bytes, const float* key_in, floa
 struct vo_split_s {
     vo_ctx ctx = nullptr;
     int n = 0, M = 0;
-    double* frag_dev = nullptr;  // [M][2 planes][n/8 row blocks][n/4 k-steps][32 lanes]
+    double* frag_dev = nullptr;  // [M][2 planes][n/8 row blocks][n/4 k-steps][32 lanes] (n >= 16)
+    std::vector<double> small_basis;  // n <= 8: the basis [M][n][n] complex interleaved, exp_small_kernel's SmallBasis parameter
     double norm1[VO_EXP_MAX_M];  // induced 1-norm of each basis matrix
     double cs[VO_EXP_MAX_M * VO_EXP_MAX_M * VO_EXP_MAX_M];
     bool has_cs = false;
@@ -157,6 +172,10 @@ int32_t launch_exp(vo_ctx c, const ExpKP& kp, const double* frag, double2* psi, 
     X(64, 1) X(64, 2) X(64, 3) X(48, 2) X(48, 3) X(40, 2) X(32, 1) X(32, 2) X(32, 3) X(32, 4) X(24, 2) X(24, 3) X(16, 1) X(16, 2) X(16, 3) X(16, 4)
 
 bool exp_geometry(int n, int M, unsigned* threads, size_t* smem) {
+    if (n >= 1 && n <= VO_EXP_SMALL_MAX_N && M >= 1 && M <= VO_EXP_MAX_M) {  // exp_small_kernel
+        *threads = VO_EXP_SMALL_THREADS, *smem = 0;
+        return true;
+    }
 #define VO_EXP_GEO(NDIM, MM) \
     if (n == NDIM && M == MM) { *threads = Geo<NDIM, MM, 16>::THREADS, *smem = Geo<NDIM, MM, 16>::SMEM; return true; }
     VO_EXP_SHAPES(VO_EXP_GEO)
@@ -167,6 +186,18 @@ bool exp_geometry(int n, int M, unsigned* threads, size_t* smem) {
 int32_t dispatch_exp(vo_split sp, const ExpKP& kp, double2* psi, double2* psi_out, const double* gp, const double2* coef_in, const CtlArrays& ca, EvSlot* ev,
                      void* custom_fn = nullptr, const int* order = nullptr, int* tile_ctr = nullptr) {
     vo_ctx c = sp->ctx;
+    if (sp->n <= VO_EXP_SMALL_MAX_N) {  // systems of 1 to 8 levels: exp_small_kernel (a per-system plan: `order` has nothing to group)
+        if (custom_fn) {
+            ExpKP kpc = kp;
+            CtlArrays cac = ca;
+            void* args[] = {&kpc, const_cast<double*>(sp->small_basis.data()), &psi, &psi_out, &gp, &coef_in, &cac, &ev};
+            int32_t r = rtc_exp_launch(c, custom_fn, exp_small_grid(c, kp.N), VO_EXP_SMALL_THREADS, 0, args);
+            if (r != VO_OK) return r;
+            VO_CHECK_LAUNCH(c);
+            return VO_OK;
+        }
+        return launch_exp_small(c, sp->n, sp->M, kp, sp->small_basis.data(), psi, psi_out, gp, coef_in, ca, ev);
+    }
     if (custom_fn) {  // the user's generator: same kernel, compiled at run time
         unsigned threads = 0;
         size_t smem = 0;
@@ -185,14 +216,14 @@ int32_t dispatch_exp(vo_split sp, const ExpKP& kp, double2* psi, double2* psi_ou
     if (sp->n == NDIM && sp->M == MM) return launch_exp<NDIM, MM, 16>(c, kp, sp->frag_dev, psi, psi_out, gp, coef_in, ca, ev, order, tile_ctr);
     VO_EXP_SHAPES(VO_EXP_CASE)
 #undef VO_EXP_CASE
-    return vo_fail(c, VO_ERR_UNSUPPORTED, "exp: the shared-basis split is compiled for n in {16, 32} with M <= 4, n in {24, 48} with M in {2, 3}, (40, 2) and n = 64 with M <= 3 "
+    return vo_fail(c, VO_ERR_UNSUPPORTED, "exp: the shared-basis split is compiled for 1 <= n <= 8 with M <= 4, n in {16, 32} with M <= 4, n in {24, 48} with M in {2, 3}, (40, 2) and n = 64 with M <= 3 "
                                           "(the whole basis stays in one SM's shared memory); other shapes: the dense split (vo_split_dense_create)");
 }
 
 ExpKP make_kp(const vo_split_s* sp, int mode) {
     ExpKP kp;
     std::memset(&kp, 0, sizeof kp);
-    kp.n = sp->n, kp.M = sp->M, kp.mode = mode, kp.taylor_deg = sp->taylor_deg;
+    kp.n = sp->n, kp.M = sp->M, kp.mode = mode, kp.taylor_deg = sp->taylor_deg, kp.n_events = 1;
     std::memcpy(kp.norm1, sp->norm1, sizeof kp.norm1);
     for (int a = 0; a < sp->M; ++a)
         for (int b = 0; b < sp->M; ++b)
@@ -281,7 +312,8 @@ __global__ void exp_group_key_kernel(const ExpKP kp, const double* __restrict__ 
 static int32_t exp_dynamic_order(vo_expsolver_s* s, const ExpKP& kp, const int** order) {
     vo_ctx c = s->ctx;
     *order = nullptr;
-    if (!s->dynamic_group || s->gen_fn || s->N < 64 || s->N > 0x7fffffff) return VO_OK;
+    // (exp_small_kernel plans every system on its own: there are no tiles to group)
+    if (!s->dynamic_group || s->gen_fn || s->sp->n <= VO_EXP_SMALL_MAX_N || s->N < 64 || s->N > 0x7fffffff) return VO_OK;
     const int n = (int)s->N;
     if (!s->key_in) {
         const size_t tmp = vo_sort_pairs_tmp_bytes(n);
@@ -300,7 +332,8 @@ static int32_t exp_dynamic_order(vo_expsolver_s* s, const ExpKP& kp, const int**
     return VO_OK;
 }
 
-int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive) {
+// One event of every system, or with events > 1 (exp_small_kernel only) that many in one launch.
+int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive, int events = 1) {
     vo_ctx c = s->ctx;
     if (adaptive && !s->want_err) return vo_fail(c, VO_ERR_NOT_ADAPTIVE, "adaptive step validation failed");  // ode.rs:312
     if (adaptive && (s->scheme == VO_EXP_MIDPOINT || s->scheme == VO_EXP_SPLIT_MIDPOINT || s->scheme == VO_EXP_SPLIT_CFM))
@@ -313,7 +346,7 @@ int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive) {
     ExpKP kp = make_kp(s->sp, 0);
     kp.M_gen = s->M_gen, kp.scheme = s->scheme, kp.adaptive = adaptive ? 1 : 0;
     kp.want_err = (s->want_err && adaptive) ? 1 : 0;  // the embedded solution only feeds the controller
-    kp.t_start = s->t0, kp.t_end = s->tf, kp.N = s->N, kp.count_events = 1;
+    kp.t_start = s->t0, kp.t_end = s->tf, kp.N = s->N, kp.count_events = 1, kp.n_events = events;
     kp.rtol = s->rtol, kp.alpha = s->alpha, kp.pw = s->pw, kp.min_dt = s->min_dt, kp.max_dt = s->max_dt;
     kp.pw_is_third = s->pw == 1.0 / 3.0;
     kp.literal_norm = (s->literal_norm && adaptive) ? 1 : 0;
@@ -355,13 +388,16 @@ int32_t exp_step_impl(vo_expsolver s, bool adaptive, vo_step_result* res) {
 extern "C" {
 
 int32_t vo_split_basis_create(vo_ctx c, int32_t n, int32_t M, const double* basis, vo_split* out) {
-    if (!c || !basis || !out || M < 1 || M > VO_EXP_MAX_M || n < 8 || n % 8) return vo_fail(c, VO_ERR_BAD_ARG, "vo_split_basis_create: need n % 8 == 0 and 1 <= M <= 4");
+    if (!c || !basis || !out || M < 1 || M > VO_EXP_MAX_M || n < 1 || (n > VO_EXP_SMALL_MAX_N && n % 8))
+        return vo_fail(c, VO_ERR_BAD_ARG, "vo_split_basis_create: need 1 <= n <= 8 or n a multiple of 8, and 1 <= M <= 4");
     DeviceGuard g(c->device);
     vo_split sp = new vo_split_s();
     sp->ctx = c, sp->n = n, sp->M = M;
     std::memset(sp->cs, 0, sizeof sp->cs);
     const int NW = n / 8, NK = n / 4;
-    std::vector<double> frag((size_t)M * 2 * n * n);
+    const bool small = n <= VO_EXP_SMALL_MAX_N;  // exp_small_kernel takes the basis as it is; the tiles of exp_step_kernel take DMMA fragments
+    std::vector<double> frag(small ? 0 : (size_t)M * 2 * n * n);
+    if (small) sp->small_basis.assign(basis, basis + (size_t)M * 2 * n * n);
     for (int m = 0; m < M; ++m) {
         double best = 0.0;  // induced 1-norm: max column sum of |B_rc|
         for (int col = 0; col < n; ++col) {
@@ -370,17 +406,19 @@ int32_t vo_split_basis_create(vo_ctx c, int32_t n, int32_t M, const double* basi
             best = std::max(best, sum);
         }
         sp->norm1[m] = best;
-        for (int p = 0; p < 2; ++p)
+        for (int p = 0; p < 2 && !small; ++p)
             for (int w = 0; w < NW; ++w)
                 for (int kk = 0; kk < NK; ++kk)
                     for (int l = 0; l < 32; ++l)  // A fragment of mma.m8n8k4: lane l holds A[l/4][l%4]
                         frag[((((size_t)(m * 2 + p) * NW + w) * NK + kk) * 32) + l] = basis[(((size_t)m * n + 8 * w + l / 4) * n + 4 * kk + l % 4) * 2 + p];
     }
-    if (vo_dmalloc(&sp->frag_dev, frag.size() * sizeof(double)) != cudaSuccess) {
-        delete sp;
-        return vo_fail(c, VO_ERR_ALLOC, "vo_split_basis_create: cudaMalloc failed");
+    if (!small) {
+        if (vo_dmalloc(&sp->frag_dev, frag.size() * sizeof(double)) != cudaSuccess) {
+            delete sp;
+            return vo_fail(c, VO_ERR_ALLOC, "vo_split_basis_create: cudaMalloc failed");
+        }
+        VO_CUDA(c, cudaMemcpyAsync(sp->frag_dev, frag.data(), frag.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     }
-    VO_CUDA(c, cudaMemcpyAsync(sp->frag_dev, frag.data(), frag.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     if (vo_dmalloc(&sp->basis_dev, sizeof(double2) * (size_t)M * n * n) != cudaSuccess) {
         vo_split_destroy(sp);
         return vo_fail(c, VO_ERR_ALLOC, "vo_split_basis_create: cudaMalloc failed");
@@ -630,9 +668,14 @@ int32_t vo_exp_run(vo_expsolver s, int32_t adaptive, int64_t max_calls, vo_step_
     int batch = 2;
     while (s->n_done < s->N && (max_calls <= 0 || calls < max_calls)) {
         int launched = 0;
-        for (int b = 0; b < batch && (max_calls <= 0 || calls < max_calls); ++b, ++calls, ++launched) {
-            int32_t r = exp_launch_event(s, adaptive != 0);
+        int left = batch;  // calls of this batch
+        if (max_calls > 0) left = (int)std::min<int64_t>(left, max_calls - calls);
+        const int fuse = s->sp->n <= VO_EXP_SMALL_MAX_N && !(s->scheme == VO_EXP_MAGNUS42 && s->dense_comm) ? VO_EXP_SMALL_FUSE : 1;
+        while (left > 0) {
+            const int ev = std::min(fuse, left);
+            int32_t r = exp_launch_event(s, adaptive != 0, ev);
             if (r != VO_OK) return r;
+            left -= ev, calls += ev, ++launched;
         }
         EvSlot d;
         int32_t r = exp_ev_read(s, &d);

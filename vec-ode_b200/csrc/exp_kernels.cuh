@@ -16,6 +16,7 @@ struct ExpKP {
     int applied_comm;     // vo_exp_set_applied_commutator: magnus_42's commutator applied to the state by products, never formed (no structure tensor)
     int literal_norm;     // vo_exp_set_literal_norm: the controller reads ca.dx_norm (= ||x0||, never rewritten) instead of ||x_err||, magnus.rs:274-276
     int nseq;             // mode 1: exponentials applied one after the other, coefficient sets [nseq][N][M]
+    int n_events;         // mode 0, exp_small_kernel: events per system and launch (vo_exp_run fuses several; exp_step_kernel runs one)
     unsigned split_mask;  // VO_EXP_SPLIT_MIDPOINT: bit m set <=> basis matrix m belongs to split A
     double t_end, t_start;
     double rtol, alpha, pw, min_dt, max_dt;
@@ -339,6 +340,200 @@ struct GenCos {
     }
 };
 
+// ---- per-system logic of one event, shared by exp_step_kernel (tiles of 16 systems on the tensor cores, n >= 16) and
+// exp_small_kernel (exp_small_kernels.cuh: one system per thread, n <= 8). Only the exponentials differ between the two.
+
+// Exponentials of an event: nbase for the propagated solution, then nerr for the embedded lower-order one (from x0).
+__device__ __forceinline__ void exp_counts_of(const ExpKP& kp, int* nbase, int* nerr) {
+    const bool tables = kp.scheme == VO_EXP_CFM4 || kp.scheme == VO_EXP_CFM_TABLE || kp.scheme == VO_EXP_SPLIT_CFM;
+    *nbase = kp.mode == 1 ? 1 : (tables ? kp.n_rows : (kp.scheme == VO_EXP_SPLIT_MIDPOINT ? 3 : 1));
+    *nerr = (kp.mode == 0 && kp.want_err) ? (tables ? kp.n_rows_err : (kp.scheme == VO_EXP_MAGNUS42 ? 1 : 0)) : 0;
+}
+
+// step_size_of (ode.rs:165-176) with t_list = [t0, tf]: the kind of this system's coming event (255: the trajectory is done) and,
+// for a step, its size dt.
+__device__ __forceinline__ int exp_event_kind(const ExpKP& kp, uint32_t word, double t, double h, double& dt) {
+    int evk = 255;
+    if (!((word >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE)) {
+        const int tgt = (int)(word & VO_WORD_TGT_MASK);
+        if (tgt >= 2) {
+            evk = VO_EV_END;
+        } else {
+            const double rem = (tgt == 0 ? kp.t_start : kp.t_end) - t;
+            if (fabs(rem) <= 2.220446049250313e-16) evk = tgt >= 1 ? VO_EV_END : VO_EV_CHKPT;
+            else dt = rem < h ? rem : h, evk = VO_EV_STEP;
+        }
+    }
+    return evk;
+}
+
+// The generator samples a step's exponents are built from (g: this system's generator parameters): midpoint at t + dt/2
+// (exp/magnus.rs:10-26); the tables at every node t + c_q dt (cfm.rs:70-72); split midpoint at t (split_exp.rs:520-562 samples
+// there, not at t + dt/2); magnus_42 at the two Gauss nodes (magnus.rs:28-83).
+template <int M, class GEN>
+__device__ __forceinline__ void exp_samples(const ExpKP& kp, const double* g, double t, double dt, double (&v)[VO_EXP_MAX_NODES][M]) {
+    if (kp.scheme == VO_EXP_MIDPOINT) {
+        GEN::template coef<M>(g, kp.M_gen, t + dt * 0.5, v[0]);
+    } else if (kp.scheme == VO_EXP_CFM4 || kp.scheme == VO_EXP_CFM_TABLE || kp.scheme == VO_EXP_SPLIT_CFM) {
+#pragma unroll
+        for (int q = 0; q < VO_EXP_MAX_NODES; ++q)
+            if (q < kp.n_nodes) GEN::template coef<M>(g, kp.M_gen, t + kp.tab_c[q] * dt, v[q]);
+    } else if (kp.scheme == VO_EXP_SPLIT_MIDPOINT) {
+        GEN::template coef<M>(g, kp.M_gen, t, v[0]);
+    } else {
+        const double c_mid = 0.288675134594812882254574390251;
+        const double b1 = dt * 0.5;
+        const double mid_t = t + b1;
+        GEN::template coef<M>(g, kp.M_gen, mid_t - c_mid * dt, v[0]);
+        GEN::template coef<M>(g, kp.M_gen, mid_t + c_mid * dt, v[1]);
+    }
+}
+
+// Exponent e of a step, exp(sum_m k[m] B_m), from the samples v (real generator coefficients, so k is real).
+//   midpoint: e = 0 only. Tables (cfm_general / split_cfm): cfm_exp (cfm.rs:31-37), k = a_0 m_0; k += a_q m_q; k *= dt, with row e of
+//   alpha (e < nbase) or of alph_err, restricted to split A or B by row_split. Split midpoint: A, B, A, each scaled by dt/2
+//   (split_exp.rs:540-559). magnus_42: 0 = w1 + w2 b2 (w1 alone with the applied commutator), 1 = w1 (the embedded solution),
+//   2 = L0, 3 = L1 (the applied commutator's two generators).
+template <int M>
+__device__ __forceinline__ void exp_row(const ExpKP& kp, int e, int nbase, const double (&v)[VO_EXP_MAX_NODES][M], double dt, double (&k)[M]) {
+    if (kp.scheme == VO_EXP_MIDPOINT) {
+#pragma unroll
+        for (int m = 0; m < M; ++m) k[m] = v[0][m] * dt;
+    } else if (kp.scheme == VO_EXP_CFM4 || kp.scheme == VO_EXP_CFM_TABLE || kp.scheme == VO_EXP_SPLIT_CFM) {
+        const double* a = e < nbase ? &kp.tab_alpha[e * VO_EXP_MAX_NODES] : &kp.tab_alpha_err[(e - nbase) * VO_EXP_MAX_NODES];
+        const int side = e < nbase ? kp.row_split[e] : 0;
+#pragma unroll
+        for (int m = 0; m < M; ++m) {
+            double s = a[0] * v[0][m];
+#pragma unroll
+            for (int q = 1; q < VO_EXP_MAX_NODES; ++q)
+                if (q < kp.n_nodes) s = s + (a[q] * v[q][m]);
+            const bool in_a = (kp.split_mask >> m) & 1u;
+            const bool keep = side == 0 || (side == 1 ? in_a : !in_a);
+            k[m] = keep ? s * dt : 0.0;
+        }
+    } else if (kp.scheme == VO_EXP_SPLIT_MIDPOINT) {
+        const double dt0 = dt * 0.5;
+#pragma unroll
+        for (int m = 0; m < M; ++m) {
+            const bool in_a = (kp.split_mask >> m) & 1u;
+            k[m] = ((e == 1) != in_a) ? v[0][m] * dt0 : 0.0;
+        }
+    } else {
+        const double b1 = dt * 0.5, b2 = dt * dt * -0.144337567297406441127287195125;
+        if (e >= 2) {
+#pragma unroll
+            for (int m = 0; m < M; ++m) k[m] = e == 2 ? v[0][m] : v[1][m];
+            return;
+        }
+        double w2[M];
+#pragma unroll
+        for (int c = 0; c < M; ++c) w2[c] = 0.0;
+        if (e == 0 && !kp.applied_comm) {
+#pragma unroll
+            for (int a = 0; a < M; ++a)
+#pragma unroll
+                for (int b = 0; b < M; ++b) {
+                    const double ab = v[0][a] * v[1][b];
+#pragma unroll
+                    for (int c = 0; c < M; ++c) {
+                        const double sc = kp.cs[(a * M + b) * M + c];
+                        if (sc != 0.0) w2[c] = w2[c] + ab * sc;
+                    }
+                }
+        }
+#pragma unroll
+        for (int m = 0; m < M; ++m) {
+            const double w1 = (v[0][m] + v[1][m]) * b1;
+            k[m] = (e == 0 && !kp.applied_comm) ? w1 + w2[m] * b2 : w1;  // u = exp(w1 + w2); u1 = exp(w1), the 2nd-order embedded solution
+        }
+    }
+}
+
+// theta = sum_m |c_m| ||B_m||_1, the bound of ||sum_m c_m B_m||_1 that the Taylor plan (taylor_plan) is made from
+template <int M, class C> __device__ __forceinline__ double exp_theta(const ExpKP& kp, C coef) {
+    double th = 0.0;
+#pragma unroll
+    for (int m = 0; m < M; ++m) {
+        const double2 c = coef(m);
+        th += hypot(c.x, c.y) * kp.norm1[m];
+    }
+    return th;
+}
+
+// The applied commutator's share of the bound: ||Omega||_1 <= ||W1||_1 + 2 |b2| ||L0||_1 ||L1||_1 (l0, l1: real coefficients)
+template <int M, class C0, class C1> __device__ __forceinline__ double exp_comm_theta(const ExpKP& kp, double dt, C0 l0, C1 l1) {
+    double n0 = 0.0, n1 = 0.0;
+#pragma unroll
+    for (int m = 0; m < M; ++m) n0 += fabs(l0(m)) * kp.norm1[m], n1 += fabs(l1(m)) * kp.norm1[m];
+    return 2.0 * (dt * dt * 0.144337567297406441127287195125) * n0 * n1;
+}
+
+// A system's control values in the solver's arrays, read and written in place.
+struct CtlAt {
+    CtlArrays ca;
+    int64_t i;
+    __device__ __forceinline__ double& t() { return ca.t[i]; }
+    __device__ __forceinline__ double& h() { return ca.h[i]; }
+    __device__ __forceinline__ double& prev_h() { return ca.prev_h[i]; }
+    __device__ __forceinline__ double& dx_norm() { return ca.dx_norm[i]; }
+    __device__ __forceinline__ uint32_t& n_accept() { return ca.n_accept[i]; }
+    __device__ __forceinline__ uint32_t& n_reject() { return ca.n_reject[i]; }
+    __device__ __forceinline__ uint32_t& word() { return ca.word[i]; }
+};
+
+struct ExpCounts {
+    unsigned step = 0, chkpt = 0, rej = 0, end = 0, stuck = 0;
+};
+
+// The end of one event of one system (phase D): for a step the controller (handle_step_adaptive, ode.rs:311-334) or the fixed-step
+// advance, for Chkpt / End checkpoint_update (ode.rs:192-195); then the status word. word and h are the values the event started
+// from, dt its step. err_norm() gives ||x_err|| and is called by the adaptive controller alone. Returns the event's final kind
+// (a step may become a rejection); only a VO_EV_STEP commits the new state.
+template <class CTL, class NRM>
+__device__ __forceinline__ int exp_event_finish(const ExpKP& kp, CTL& c, int evk, uint32_t word, double h, double dt, NRM err_norm, ExpCounts& cnt) {
+    int tgt = (int)(word & VO_WORD_TGT_MASK);
+    uint32_t status = word >> VO_WORD_STATUS_SHIFT;
+    if (evk == VO_EV_STEP) {
+        if (kp.adaptive) {
+            const double dxn = kp.literal_norm ? c.dx_norm() : err_norm();
+            const double f = kp.rtol / dxn;
+            const double mul = step_size_mul<true>(kp.alpha, f, kp.pw, kp.pw_is_third);  // ode.rs:133-135, powf correctly rounded (rk_small.cuh)
+            const double fp_lim = at_most(at_least(mul, 0.3), 2.0);
+            const double new_h = at_most(at_least(fp_lim * h, kp.min_dt), kp.max_dt);
+            if (!(dxn == dxn)) status |= VO_TRAJ_NONFINITE;
+            if (f <= 1.0) {
+                evk = VO_EV_REJECT;
+                if (h <= kp.min_dt) status |= VO_TRAJ_STUCK, ++cnt.stuck;
+            }
+            c.prev_h() = h, c.h() = new_h, c.dx_norm() = dxn;
+        }
+        if (evk == VO_EV_STEP) c.t() += dt, c.n_accept() += 1, ++cnt.step;
+        else c.n_reject() += 1, ++cnt.rej;
+    } else {  // Chkpt / End
+        tgt += 1, c.h() = c.prev_h();
+        if (evk == VO_EV_END) status |= VO_TRAJ_DONE, ++cnt.end;
+        else ++cnt.chkpt;
+    }
+    const uint32_t nw = ((uint32_t)tgt & VO_WORD_TGT_MASK) | (status << VO_WORD_STATUS_SHIFT);
+    if (nw != word) c.word() = nw;
+    return evk;
+}
+
+// The event counters of one warp (all 32 lanes call), added to one of the VO_EV_SLOTS slots by lane 0.
+__device__ __forceinline__ void exp_counts_flush(EvSlot* slot, ExpCounts cnt) {
+    cnt.step = __reduce_add_sync(0xffffffffu, cnt.step), cnt.chkpt = __reduce_add_sync(0xffffffffu, cnt.chkpt);
+    cnt.rej = __reduce_add_sync(0xffffffffu, cnt.rej), cnt.end = __reduce_add_sync(0xffffffffu, cnt.end);
+    cnt.stuck = __reduce_add_sync(0xffffffffu, cnt.stuck);
+    if ((threadIdx.x & 31) == 0) {
+        if (cnt.step) atomicAdd(&slot->n_step, (unsigned long long)cnt.step);
+        if (cnt.chkpt) atomicAdd(&slot->n_chkpt, (unsigned long long)cnt.chkpt);
+        if (cnt.rej) atomicAdd(&slot->n_reject, (unsigned long long)cnt.rej);
+        if (cnt.end) atomicAdd(&slot->n_end, (unsigned long long)cnt.end);
+        if (cnt.stuck) atomicAdd(&slot->n_stuck, (unsigned long long)cnt.stuck);
+    }
+}
+
 template <int NDIM, int M, int TB, class GEN>
 __global__ void __launch_bounds__(Geo<NDIM, M, TB>::THREADS, 1)
 exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ frag, double2* __restrict__ psi, double2* __restrict__ psi_out,
@@ -367,7 +562,7 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
 
     const int64_t n_tiles = (kp.N + TB - 1) / TB;
     int buf = 0;
-    unsigned c_step = 0, c_chkpt = 0, c_rej = 0, c_end = 0, c_stuck = 0;
+    ExpCounts cnt;
     // Tile -> slots. With the dynamic grouping the slots are sorted by ascending theta, so tiles differ in cost: they are then taken from
     // the expensive end and handed out by an atomic counter as CTAs become free (longest-processing-time-first), which also removes the
     // 42-or-43-tiles-per-CTA quantisation of a static stride. Without it: the static stride.
@@ -402,10 +597,8 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
         const int64_t base = tile_base(tile);
         uint32_t a_word = 0;  // this slot's status word and step size, from phase A to phase D (same thread)
         double a_h = 0.0;
-        // exponentials of this event: nbase for the propagated solution, then nerr for the embedded lower-order one (from x0)
-        const bool tables = kp.scheme == VO_EXP_CFM4 || kp.scheme == VO_EXP_CFM_TABLE || kp.scheme == VO_EXP_SPLIT_CFM;
-        const int nbase = kp.mode == 1 ? 1 : (tables ? kp.n_rows : (kp.scheme == VO_EXP_SPLIT_MIDPOINT ? 3 : 1));
-        const int nerr = (kp.mode == 0 && kp.want_err) ? (tables ? kp.n_rows_err : (kp.scheme == VO_EXP_MAGNUS42 ? 1 : 0)) : 0;
+        int nbase, nerr;
+        exp_counts_of(kp, &nbase, &nerr);
         const int nexp = nbase + nerr;
         // ---- phase A: per-system control and exponent coefficients (one thread per system), written straight to shared memory
         if (threadIdx.x < TB) {
@@ -436,107 +629,26 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
 #pragma unroll
                     for (int m = 0; m < M; ++m) sCoef[m * TB + s] = coef_in[sys * M + m];
                 } else {
-                    const uint32_t word = a_word;
-                    if (!((word >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE)) {
-                        const int tgt = (int)(word & VO_WORD_TGT_MASK);
-                        const double t = a_t, h = a_h;
-                        // step_size_of (ode.rs:165-176) with t_list = [t0, tf]
-                        if (tgt >= 2) {
-                            evk = VO_EV_END;
-                        } else {
-                            const double rem = (tgt == 0 ? kp.t_start : kp.t_end) - t;
-                            if (fabs(rem) <= 2.220446049250313e-16) evk = tgt >= 1 ? VO_EV_END : VO_EV_CHKPT;
-                            else dt = rem < h ? rem : h, evk = VO_EV_STEP;
-                        }
-                        if (evk == VO_EV_STEP) {
-                            const double* g = a_g;  // this system's generator parameters (prefetched)
-                            if (kp.scheme == VO_EXP_MIDPOINT) {  // exp/magnus.rs:10-26
-                                double l[M];
-                                GEN::template coef<M>(g, kp.M_gen, t + dt * 0.5, l);
+                    evk = exp_event_kind(kp, a_word, a_t, a_h, dt);
+                    if (evk == VO_EV_STEP) {
+                        double v[VO_EXP_MAX_NODES][M];
+                        exp_samples<M, GEN>(kp, a_g, a_t, dt, v);
+                        for (int e = 0; e < (kp.applied_comm ? 4 : nexp); ++e) {
+                            double k[M];
+                            exp_row<M>(kp, e, nbase, v, dt, k);
 #pragma unroll
-                                for (int m = 0; m < M; ++m) put(0, m, l[m] * dt, 0.0);
-                            } else if (tables) {
-                                // cfm_general (exp/cfm.rs:43-100) / split_cfm (exp/split_exp.rs:568-609): the generator at every node
-                                // (cfm.rs:70-72), then per exponential cfm_exp (cfm.rs:31-37): k = a_0 m_0; k += a_q m_q; k *= dt
-                                double v[VO_EXP_MAX_NODES][M];
-#pragma unroll
-                                for (int q = 0; q < VO_EXP_MAX_NODES; ++q)
-                                    if (q < kp.n_nodes) GEN::template coef<M>(g, kp.M_gen, t + kp.tab_c[q] * dt, v[q]);
-                                for (int e = 0; e < nexp; ++e) {
-                                    const double* a = e < nbase ? &kp.tab_alpha[e * VO_EXP_MAX_NODES] : &kp.tab_alpha_err[(e - nbase) * VO_EXP_MAX_NODES];
-                                    const int side = e < nbase ? kp.row_split[e] : 0;
-#pragma unroll
-                                    for (int m = 0; m < M; ++m) {
-                                        double k = a[0] * v[0][m];
-#pragma unroll
-                                        for (int q = 1; q < VO_EXP_MAX_NODES; ++q)
-                                            if (q < kp.n_nodes) k = k + (a[q] * v[q][m]);
-                                        const bool in_a = (kp.split_mask >> m) & 1u;
-                                        const bool keep = side == 0 || (side == 1 ? in_a : !in_a);
-                                        put(e, m, keep ? k * dt : 0.0, 0.0);
-                                    }
-                                }
-                            } else if (kp.scheme == VO_EXP_SPLIT_MIDPOINT) {  // split_exp_midpoint, exp/split_exp.rs:520-562
-                                // literal: the generator is sampled at t (not t + dt/2) and BOTH splits are scaled by dt/2
-                                // (KA[0] and KB[0] by dt0, :540-548), applied as A, B, A (:556-559)
-                                double l[M];
-                                GEN::template coef<M>(g, kp.M_gen, t, l);
-                                const double dt0 = dt * 0.5;
-#pragma unroll
-                                for (int m = 0; m < M; ++m) {
-                                    const bool in_a = (kp.split_mask >> m) & 1u;
-                                    put(0, m, in_a ? l[m] * dt0 : 0.0, 0.0);
-                                    put(1, m, in_a ? 0.0 : l[m] * dt0, 0.0);
-                                    put(2, m, in_a ? l[m] * dt0 : 0.0, 0.0);
-                                }
-                            } else {  // magnus_42, exp/magnus.rs:28-83
-                                const double c_mid = 0.288675134594812882254574390251;
-                                const double b1 = dt * 0.5, b2 = dt * dt * -0.144337567297406441127287195125;
-                                const double mid_t = t + b1;
-                                double l0[M], l1[M], w2[M];
-                                GEN::template coef<M>(g, kp.M_gen, mid_t - c_mid * dt, l0);
-                                GEN::template coef<M>(g, kp.M_gen, mid_t + c_mid * dt, l1);
-#pragma unroll
-                                for (int c = 0; c < M; ++c) w2[c] = 0.0;
-#pragma unroll
-                                for (int a = 0; a < M; ++a)
-#pragma unroll
-                                    for (int b = 0; b < M; ++b) {
-                                        const double ab = l0[a] * l1[b];
-#pragma unroll
-                                        for (int c = 0; c < M; ++c) {
-                                            const double sc = kp.cs[(a * M + b) * M + c];
-                                            if (sc != 0.0) w2[c] = w2[c] + ab * sc;
-                                        }
-                                    }
-#pragma unroll
-                                for (int m = 0; m < M; ++m) {
-                                    const double w1 = (l0[m] + l1[m]) * b1;
-                                    put(0, m, kp.applied_comm ? w1 : w1 + w2[m] * b2, 0.0);  // u = exp(w1 + w2) (applied: w2 never formed)
-                                    if (nerr) put(1, m, w1, 0.0);     // u1 = exp(w1), the 2nd-order embedded solution
-                                    if (kp.applied_comm) put(2, m, l0[m], 0.0), put(3, m, l1[m], 0.0);
-                                }
-                            }
+                            for (int m = 0; m < M; ++m) put(e, m, k[m], 0.0);
                         }
                     }
                 }
             }
             sEv[s] = evk, sDt[s] = dt;
             for (int e = 0; e < nexp; ++e) {
-                double th = 0.0;
-#pragma unroll
-                for (int m = 0; m < M; ++m) {
-                    const double2 c = sCoef[(e * M + m) * TB + s];
-                    th += hypot(c.x, c.y) * kp.norm1[m];
-                }
+                const double th = exp_theta<M>(kp, [&](int m) { return sCoef[(e * M + m) * TB + s]; });
                 sTheta[e * TB + s] = evk == VO_EV_STEP ? th : 0.0;
             }
-            if (kp.applied_comm && kp.scheme == VO_EXP_MAGNUS42 && kp.mode == 0 && evk == VO_EV_STEP) {  // ||Omega||_1 <= ||W1|| + 2 |b2| ||L0|| ||L1||
-                double n0 = 0.0, n1 = 0.0;
-#pragma unroll
-                for (int m = 0; m < M; ++m) n0 += fabs(sCoef[(2 * M + m) * TB + s].x) * kp.norm1[m], n1 += fabs(sCoef[(3 * M + m) * TB + s].x) * kp.norm1[m];
-                sTheta[s] += 2.0 * (dt * dt * 0.144337567297406441127287195125) * n0 * n1;
-            }
+            if (kp.applied_comm && kp.scheme == VO_EXP_MAGNUS42 && kp.mode == 0 && evk == VO_EV_STEP)
+                sTheta[s] += exp_comm_theta<M>(kp, dt, [&](int m) { return sCoef[(2 * M + m) * TB + s].x; }, [&](int m) { return sCoef[(3 * M + m) * TB + s].x; });
         }
         __syncthreads();
         // ---- phase B: tile-uniform Taylor plan, one thread per exponential
@@ -629,42 +741,18 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
                 const int s = threadIdx.x;
                 const int64_t sys = sSys[s];
                 int evk = sEv[s];
-                if (evk != 255) {
-                    const uint32_t word = a_word;  // read in phase A by this thread; nothing has written it since
-                    int tgt = (int)(word & VO_WORD_TGT_MASK);
-                    uint32_t status = word >> VO_WORD_STATUS_SHIFT;
-                    if (evk == VO_EV_STEP) {
-                        const double h = a_h;
-                        if (kp.adaptive) {  // handle_step_adaptive, ode.rs:311-334
-                            double nn = 0.0;
+                if (evk != 255) {  // a_word, a_h: read in phase A by this thread; nothing has written them since
+                    CtlAt c{ca, sys};
+                    sEv[s] = exp_event_finish(kp, c, evk, a_word, a_h, sDt[s], [&]() {
+                        double nn = 0.0;
 #ifdef VO_USER_NORM
-                            for (int ww = 0; ww < G::NW; ++ww) nn = vo_user_join(nn, sNorm[ww * TB + s]);
-                            const double dxn = kp.literal_norm ? ca.dx_norm[sys] : VoUserNorm::finish(nn, NDIM);
+                        for (int ww = 0; ww < G::NW; ++ww) nn = vo_user_join(nn, sNorm[ww * TB + s]);
+                        return VoUserNorm::finish(nn, NDIM);
 #else
-                            for (int ww = 0; ww < G::NW; ++ww) nn += sNorm[ww * TB + s];
-                            const double dxn = kp.literal_norm ? ca.dx_norm[sys] : sqrt(nn);
+                        for (int ww = 0; ww < G::NW; ++ww) nn += sNorm[ww * TB + s];
+                        return sqrt(nn);
 #endif
-                            const double f = kp.rtol / dxn;
-                            const double mul = step_size_mul<true>(kp.alpha, f, kp.pw, kp.pw_is_third);  // ode.rs:133-135, powf correctly rounded (rk_small.cuh)
-                            const double fp_lim = at_most(at_least(mul, 0.3), 2.0);
-                            const double new_h = at_most(at_least(fp_lim * h, kp.min_dt), kp.max_dt);
-                            if (!(dxn == dxn)) status |= VO_TRAJ_NONFINITE;
-                            if (f <= 1.0) {
-                                evk = VO_EV_REJECT;
-                                if (h <= kp.min_dt) status |= VO_TRAJ_STUCK, ++c_stuck;
-                            }
-                            ca.prev_h[sys] = h, ca.h[sys] = new_h, ca.dx_norm[sys] = dxn;
-                        }
-                        if (evk == VO_EV_STEP) ca.t[sys] += sDt[s], ca.n_accept[sys] += 1, ++c_step;
-                        else ca.n_reject[sys] += 1, ++c_rej;
-                    } else {  // Chkpt / End: checkpoint_update, ode.rs:192-195
-                        tgt += 1, ca.h[sys] = ca.prev_h[sys];
-                        if (evk == VO_EV_END) status |= VO_TRAJ_DONE, ++c_end;
-                        else ++c_chkpt;
-                    }
-                    const uint32_t nw = ((uint32_t)tgt & VO_WORD_TGT_MASK) | (status << VO_WORD_STATUS_SHIFT);
-                    if (nw != word) ca.word[sys] = nw;
-                    sEv[s] = evk;
+                    }, cnt);
                 }
             }
             __syncthreads();
@@ -683,17 +771,5 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
         }
         __syncthreads();  // sEv / sCoef are rewritten by the next tile
     }
-    if (kp.mode == 0 && kp.count_events && threadIdx.x < 32) {
-        c_step = __reduce_add_sync(0xffffffffu, c_step), c_chkpt = __reduce_add_sync(0xffffffffu, c_chkpt);
-        c_rej = __reduce_add_sync(0xffffffffu, c_rej), c_end = __reduce_add_sync(0xffffffffu, c_end);
-        c_stuck = __reduce_add_sync(0xffffffffu, c_stuck);
-        if (threadIdx.x == 0) {
-            EvSlot* slot = ev + (blockIdx.x % VO_EV_SLOTS);
-            if (c_step) atomicAdd(&slot->n_step, (unsigned long long)c_step);
-            if (c_chkpt) atomicAdd(&slot->n_chkpt, (unsigned long long)c_chkpt);
-            if (c_rej) atomicAdd(&slot->n_reject, (unsigned long long)c_rej);
-            if (c_end) atomicAdd(&slot->n_end, (unsigned long long)c_end);
-            if (c_stuck) atomicAdd(&slot->n_stuck, (unsigned long long)c_stuck);
-        }
-    }
+    if (kp.mode == 0 && kp.count_events && threadIdx.x < 32) exp_counts_flush(ev + (blockIdx.x % VO_EV_SLOTS), cnt);
 }

@@ -452,7 +452,8 @@ void custom_rhs_release(vo_rhs_s* r) {
 // The functor wraps statements that assign g[1] .. g[M_gen-1], the real coefficients of L(t) = B_0 + sum_m g[m] B_m, from the
 // time `t` and this system's parameter row `p` (the 3 (M_gen - 1) doubles per system handed to vo_exp_create).
 int32_t rtc_exp_compile(const std::string& body, const std::string& norm_src, int ndim, int M, std::vector<char>& cubin, std::string& lowered, std::string& log) {
-    std::string src = norm_src + "#include \"exp_kernels.cuh\"\n";
+    const bool small = ndim <= VO_EXP_SMALL_MAX_N;  // exp_small_kernel for 1 <= n <= 8, the tensor-core tiles above
+    std::string src = norm_src + (small ? "#include \"exp_small_kernels.cuh\"\n" : "#include \"exp_kernels.cuh\"\n");
     const bool user_gen = !body.empty();
     if (user_gen)
         src += "struct GenCustom {\n"
@@ -460,7 +461,8 @@ int32_t rtc_exp_compile(const std::string& body, const std::string& norm_src, in
                "        double g[M];\n#pragma unroll\n        for (int m = 0; m < M; ++m) g[m] = 0.0;\n        {\n#line 1 \"generator_body\"\n" +
                body +
                "\n        }\n#pragma unroll\n        for (int m = 0; m < M; ++m) c[m] = (m >= 1 && m < M_gen) ? g[m] : 0.0;\n        c[0] = 1.0;\n    }\n};\n";
-    std::vector<std::string> names = {"exp_step_kernel<" + std::to_string(ndim) + ", " + std::to_string(M) + ", 16, " + (user_gen ? "GenCustom" : "GenCos") + ">"}, low;
+    const std::string shape = std::to_string(ndim) + ", " + std::to_string(M) + (small ? ", " : ", 16, ");
+    std::vector<std::string> names = {(small ? "exp_small_kernel<" : "exp_step_kernel<") + shape + (user_gen ? "GenCustom" : "GenCos") + ">"}, low;
     const int32_t rc = rtc_compile(src, names, false, cubin, low, log);
     if (rc == VO_OK) lowered = low[0];
     return rc;
@@ -650,7 +652,10 @@ int32_t vo_normfn_check_kernels(const char* map_body, int32_t join, const char* 
     if (rc == VO_OK && exp_n > 0) {
         std::vector<char> cubin;
         std::string lowered;
-        rc = rtc_exp_compile("", norm_source(&f), exp_n, exp_M, cubin, lowered, msg);
+        if (exp_n > 64 || (exp_n > VO_EXP_SMALL_MAX_N && exp_n % 8) || exp_M < 1 || exp_M > 4)
+            rc = VO_ERR_BAD_ARG, msg = "vo_normfn_check_kernels: exp_n must be 1 <= n <= 8 or a multiple of 8 up to 64, and 1 <= exp_M <= 4";
+        else
+            rc = rtc_exp_compile("", norm_source(&f), exp_n, exp_M, cubin, lowered, msg);
         total += cubin.size();
     }
     if (rc != VO_OK) {
@@ -681,7 +686,8 @@ int32_t vo_norm_custom(vo_ens e, vo_normfn f, double* out_host) {
 
 int32_t vo_exp_generator_check(const char* body, int32_t n, int32_t M, char* log, int64_t log_cap) {
     if (log && log_cap > 0) log[0] = '\0';
-    if (!body || n < 8 || n > 64 || n % 8 || M < 1 || M > 4) return vo_fail(nullptr, VO_ERR_BAD_ARG, "vo_exp_generator_check: bad argument");
+    if (!body || n < 1 || n > 64 || (n > VO_EXP_SMALL_MAX_N && n % 8) || M < 1 || M > 4)
+        return vo_fail(nullptr, VO_ERR_BAD_ARG, "vo_exp_generator_check: need 1 <= n <= 8 or n a multiple of 8 up to 64, and 1 <= M <= 4");
     std::vector<char> cubin;
     std::string lowered, msg;
     const int32_t rc = rtc_exp_compile(body, "", n, M, cubin, lowered, msg);

@@ -25,7 +25,11 @@ _vp = C.c_void_p
 
 
 class DenseBasisSplit:
-    """ExponentialSplit (+ Commutator, NormedExponentialSplit) for batched dense complex systems on a shared basis."""
+    """ExponentialSplit (+ Commutator, NormedExponentialSplit) for batched dense complex systems on a shared basis.
+
+    `basis`: [M][n][n] complex, 1 <= M <= 4, with 1 <= n <= 8 (qubits, qutrits, few-qubit registers: one system per GPU thread in
+    FP64 registers, each with its own Taylor plan; vo_exp_run fuses several events per launch) or n a multiple of 8 (16 to 64 on the
+    FP64 tensor cores, by tiles of 16 systems). 9 <= n <= 15 is refused."""
 
     def __init__(self, ctx: Context, basis, commutator_structure=None, taylor_degree: int = 0):
         basis = np.ascontiguousarray(basis, dtype=np.complex128)
