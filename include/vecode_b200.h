@@ -441,6 +441,23 @@ int32_t vo_exp_stats(vo_expsolver s, int64_t* accepted, int64_t* rejected, doubl
 /* Back to (t0, psi0, h): psi0_host NULL re-uses the state given at creation, otherwise uploads a new one. */
 int32_t vo_exp_reset(vo_expsolver s, const double* psi0_host);
 void* vo_exp_state_device_ptr(vo_expsolver s);
+/* Output times: the pub field ODEData.t_list (ode.rs:89-90) in place of [t0, tf] (ode.rs:144), as vo_solver_set_t_list. Steps are
+ * clipped to land on every entry (step_size_of / check_step, ode.rs:165-176, 389-399); each system raises Chkpt at every entry
+ * before the last and End at the last (ode.rs:192-195), in whatever call it gets there under adaptive control. 1 <= n <= 65535
+ * entries (VO_ERR_UNSUPPORTED above, VO_ERR_BAD_ARG for n < 1 or NULL). Refused with VO_ERR_STATE once a step / run has begun;
+ * vo_exp_reset rewinds every system to entry 0 and accepts a new list. */
+int32_t vo_exp_set_t_list(vo_expsolver s, const double* t_list, int32_t n);
+/* Checkpoint output: keep, for every entry k of t_list, the state each system shows through vo_exp_current at its Chkpt / End event
+ * for t_list[k] (the kernels write it at the event, also in the middle of a fused vo_exp_run launch). Storage [len][N][n] complex,
+ * zeroed when enabled and re-allocated by vo_exp_set_t_list; vo_exp_reset keeps the contents until the next run overwrites them.
+ * Snapshot k is complete once every system has passed t_list[k] (vo_exp_stats' t tells). Both readers speak the caller's order
+ * (vo_exp_set_order: the kernels write each system to its caller's row) and return VO_ERR_BAD_ARG for k outside the list and
+ * VO_ERR_STATE when snapshots are off. vo_exp_snapshot copies [N][n] (re, im) to the host; vo_exp_snapshot_device returns a
+ * non-owning device view of one row of 2 n N doubles (destroy it with vo_ens_destroy; the storage belongs to the solver), what
+ * vo_group_gather_placed takes. */
+int32_t vo_exp_enable_snapshots(vo_expsolver s);
+int32_t vo_exp_snapshot(vo_expsolver s, int32_t k, double* psi_host /* [N][n] (re,im) */);
+int32_t vo_exp_snapshot_device(vo_expsolver s, int32_t k, vo_ens* out);
 
 /* ---- multi-GPU: one ensemble sharded by trajectory over the GPUs of one box ------------------------------------------ */
 /* The reference has no parallelism of any kind; what replaces "one solver object per trajectory, run them in any order" is

@@ -183,6 +183,10 @@ SIGNATURES = {
     "vo_exp_stats": (_i32, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "vo_exp_reset": (_i32, [_vp, _vp]),
     "vo_exp_state_device_ptr": (_vp, [_vp]),
+    "vo_exp_set_t_list": (_i32, [_vp, _vp, _i32]),
+    "vo_exp_enable_snapshots": (_i32, [_vp]),
+    "vo_exp_snapshot": (_i32, [_vp, _i32, _vp]),
+    "vo_exp_snapshot_device": (_i32, [_vp, _i32, _pvp]),
     "vo_group_unique_id": (_i32, [_vp]),
     "vo_group_create_rank": (_i32, [_vp, _vp, _i32, _i32, _pvp]),
     "vo_group_create_local": (_i32, [_pvp, _i32, _pvp]),

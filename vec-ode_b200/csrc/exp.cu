@@ -70,6 +70,10 @@ struct vo_expsolver_s {
     EvSlot* ev_host = nullptr;
     EvSlot ev_seen{};
     int64_t n_done = 0;
+    std::vector<double> t_list;   // ODEData.t_list (ode.rs:89): [t0, tf] (ode.rs:144) unless vo_exp_set_t_list
+    double* t_list_dev = nullptr;  // device copy of a list longer than VO_INLINE_TLIST
+    double2* snap = nullptr;       // [t_list.size()][N][n] in the caller's order (vo_exp_enable_snapshots), else NULL
+    bool stepped = false;          // an event has run since creation or the last vo_exp_reset: the list is fixed until the next reset
     bool want_err = true;  // alph_err / x_err present (exp/cfm.rs:157-161)
     unsigned split_mask = 1u;  // VO_EXP_SPLIT_MIDPOINT: which basis matrices form split A (default: B_0)
     double atol = 1.0e-6, rtol = 1.0e-4, alpha = 0.9, pw = 1.0 / 3.0, min_dt = 1.0e-6, max_dt = 1.0;
@@ -346,7 +350,10 @@ int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive, int events = 1) {
     ExpKP kp = make_kp(s->sp, 0);
     kp.M_gen = s->M_gen, kp.scheme = s->scheme, kp.adaptive = adaptive ? 1 : 0;
     kp.want_err = (s->want_err && adaptive) ? 1 : 0;  // the embedded solution only feeds the controller
-    kp.t_start = s->t0, kp.t_end = s->tf, kp.N = s->N, kp.count_events = 1, kp.n_events = events;
+    kp.N = s->N, kp.count_events = 1, kp.n_events = events;
+    kp.n_tlist = (int)s->t_list.size(), kp.t_list = s->t_list_dev;
+    for (int i = 0; i < VO_INLINE_TLIST && i < kp.n_tlist; ++i) kp.t_list_inline[i] = s->t_list[i];
+    kp.snap = s->snap, kp.snap_perm = s->perm;
     kp.rtol = s->rtol, kp.alpha = s->alpha, kp.pw = s->pw, kp.min_dt = s->min_dt, kp.max_dt = s->max_dt;
     kp.pw_is_third = s->pw == 1.0 / 3.0;
     kp.literal_norm = (s->literal_norm && adaptive) ? 1 : 0;
@@ -355,6 +362,7 @@ int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive, int events = 1) {
     kp.n_nodes = s->n_nodes, kp.n_rows = s->n_rows, kp.n_rows_err = s->n_rows_err;
     std::memcpy(kp.tab_c, s->tab_c, sizeof kp.tab_c), std::memcpy(kp.tab_alpha, s->tab_alpha, sizeof kp.tab_alpha);
     std::memcpy(kp.tab_alpha_err, s->tab_alpha_err, sizeof kp.tab_alpha_err), std::memcpy(kp.row_split, s->row_split, sizeof kp.row_split);
+    s->stepped = true;
     if (s->scheme == VO_EXP_MAGNUS42 && s->dense_comm) return launch_magnus_dense(s, kp);
     const int* order = nullptr;
     int32_t orc = exp_dynamic_order(s, kp, &order);
@@ -520,6 +528,7 @@ int32_t vo_exp_create(vo_ctx c, vo_split sp, int32_t scheme, int32_t M_gen, cons
     DeviceGuard g(c->device);
     vo_expsolver s = new vo_expsolver_s();
     s->ctx = c, s->sp = sp, s->scheme = scheme, s->M_gen = M_gen, s->N = N, s->t0 = t0, s->tf = tf, s->h_init = h;
+    s->t_list = {t0, tf};  // ODEData::new, ode.rs:144
     if (scheme == VO_EXP_CFM4) exp_store_tables(s, C_GAUSS_LEGENDRE_4, 2, CFM_R4_J2_GL, 2, CFM_R2_J1_GL, 1);  // ExpCFMSolver::new, cfm.rs:131-154
     const size_t nb = sizeof(double2) * (size_t)N * sp->n, ngp = sizeof(double) * (size_t)N * std::max(1, M_gen - 1) * 3;
     bool ok = vo_dmalloc(&s->psi, nb) == cudaSuccess && vo_dmalloc(&s->psi0, nb) == cudaSuccess && vo_dmalloc(&s->gp, ngp) == cudaSuccess &&
@@ -552,7 +561,19 @@ int32_t vo_exp_destroy(vo_expsolver s) {
     vo_dfree(s->ev_dev), cudaFreeHost(s->ev_host);
     rtc_exp_unload(s->gen_module);
     vo_dfree(s->perm), vo_dfree(s->stage);
+    vo_dfree(s->t_list_dev), vo_dfree(s->snap);
     delete s;
+    return VO_OK;
+}
+
+// Snapshot storage for the current list, zeroed: a system writes its row of entry k at its Chkpt / End event for t_list[k]
+static int32_t exp_alloc_snapshots(vo_expsolver_s* s) {
+    vo_ctx c = s->ctx;
+    VO_CUDA(c, cudaStreamSynchronize(c->stream));
+    vo_dfree(s->snap), s->snap = nullptr;
+    const size_t bytes = sizeof(double2) * s->t_list.size() * (size_t)s->N * s->sp->n;
+    if (vo_dmalloc(&s->snap, bytes) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "vo_exp_enable_snapshots: cudaMalloc failed");
+    VO_CUDA(c, cudaMemsetAsync(s->snap, 0, bytes, c->stream));
     return VO_OK;
 }
 
@@ -789,7 +810,7 @@ int32_t vo_exp_reset(vo_expsolver s, const double* psi0_host) {
     VO_CUDA(c, cudaMemcpyAsync(s->psi, s->psi0, nb, cudaMemcpyDeviceToDevice, c->stream));
     VO_CUDA(c, cudaMemsetAsync(s->ev_dev, 0, sizeof(EvSlot) * VO_EV_SLOTS, c->stream));
     std::memset(&s->ev_seen, 0, sizeof s->ev_seen);
-    s->n_done = 0;
+    s->n_done = 0, s->stepped = false;
     exp_ctl_fill_kernel<<<(unsigned)ceil_div(s->N, 256), 256, 0, c->stream>>>(s->ca, s->N, s->t0, s->h_init);
     VO_CHECK_LAUNCH(c);
     if (s->literal_norm) return exp_fill_literal_norm(s);
@@ -822,6 +843,55 @@ int32_t vo_exp_set_order(vo_expsolver s, const int64_t* perm, int64_t n) {
 }
 
 void* vo_exp_state_device_ptr(vo_expsolver s) { return s ? (void*)s->psi : nullptr; }
+
+int32_t vo_exp_set_t_list(vo_expsolver s, const double* t_list, int32_t n) {
+    if (!s || !t_list || n < 1) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_set_t_list: bad argument");
+    if (n > (int32_t)VO_WORD_TGT_MASK) return vo_fail(s->ctx, VO_ERR_UNSUPPORTED, "vo_exp_set_t_list: list too long for per-system control");
+    if (s->stepped) return vo_fail(s->ctx, VO_ERR_STATE, "vo_exp_set_t_list: stepping has begun (vo_exp_reset rewinds it)");
+    vo_ctx c = s->ctx;
+    DeviceGuard g(c->device);
+    VO_CUDA(c, cudaStreamSynchronize(c->stream));
+    vo_dfree(s->t_list_dev), s->t_list_dev = nullptr;
+    if (n > VO_INLINE_TLIST) {
+        if (vo_dmalloc(&s->t_list_dev, sizeof(double) * n) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "vo_exp_set_t_list: cudaMalloc failed");
+        VO_CUDA(c, cudaMemcpy(s->t_list_dev, t_list, sizeof(double) * n, cudaMemcpyHostToDevice));
+    }
+    s->t_list.assign(t_list, t_list + n);
+    return s->snap ? exp_alloc_snapshots(s) : VO_OK;
+}
+
+int32_t vo_exp_enable_snapshots(vo_expsolver s) {
+    if (!s) return VO_ERR_BAD_ARG;
+    if (s->snap) return VO_OK;
+    DeviceGuard g(s->ctx->device);
+    return exp_alloc_snapshots(s);
+}
+
+static int32_t exp_snapshot_check(vo_expsolver s, int32_t k) {
+    if (!s->snap) return vo_fail(s->ctx, VO_ERR_STATE, "vo_exp_snapshot: snapshots are not enabled (vo_exp_enable_snapshots)");
+    if (k < 0 || k >= (int32_t)s->t_list.size()) return vo_fail(s->ctx, VO_ERR_BAD_ARG, "vo_exp_snapshot: index outside t_list");
+    return VO_OK;
+}
+
+int32_t vo_exp_snapshot(vo_expsolver s, int32_t k, double* psi_host) {
+    if (!s || !psi_host) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_snapshot: NULL argument");
+    int32_t r = exp_snapshot_check(s, k);
+    if (r != VO_OK) return r;
+    vo_ctx c = s->ctx;
+    DeviceGuard g(c->device);
+    const size_t row = (size_t)s->N * s->sp->n;
+    VO_CUDA(c, cudaMemcpyAsync(psi_host, s->snap + (size_t)k * row, sizeof(double2) * row, cudaMemcpyDeviceToHost, c->stream));
+    VO_CUDA(c, cudaStreamSynchronize(c->stream));
+    return VO_OK;
+}
+
+int32_t vo_exp_snapshot_device(vo_expsolver s, int32_t k, vo_ens* out) {
+    if (!s || !out) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_snapshot_device: NULL argument");
+    int32_t r = exp_snapshot_check(s, k);
+    if (r != VO_OK) return r;
+    const int64_t row = (int64_t)s->N * s->sp->n;
+    return vo_ens_wrap(s->ctx, s->snap + (size_t)k * row, 1, 2 * row, out);
+}
 
 
 // ---- dense split: ExponentialSplit / Commutator / NormedExponentialSplit (exp/mod.rs:11-54) with per-system n x n operators ------

@@ -247,29 +247,19 @@ __global__ void __launch_bounds__(32 * NB) magnus_dense_kernel(const __grid_cons
         __syncthreads();
         // ---- control: step_size_of (ode.rs:165-176), generator coefficients at the two nodes (magnus.rs:42-52)
         if (threadIdx.x == 0) {
-            int evk = 255;
             double dt = 0.0;
             const uint32_t word = ca.word[sys];
-            if (!((word >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE)) {
-                const int tgt = (int)(word & VO_WORD_TGT_MASK);
-                const double t = ca.t[sys], h = ca.h[sys];
-                if (tgt >= 2) {
-                    evk = VO_EV_END;
-                } else {
-                    const double rem = (tgt == 0 ? kp.t_start : kp.t_end) - t;
-                    if (fabs(rem) <= 2.220446049250313e-16) evk = tgt >= 1 ? VO_EV_END : VO_EV_CHKPT;
-                    else dt = rem < h ? rem : h, evk = VO_EV_STEP;
-                }
-                if (evk == VO_EV_STEP) {
-                    const double c_mid = 0.288675134594812882254574390251;
-                    const double mid_t = t + dt * 0.5;
-                    double g0[MMAX], g1[MMAX];
-                    GEN::template coef<MMAX>(gp + sys * (kp.M_gen - 1) * 3, kp.M_gen, mid_t - c_mid * dt, g0);
-                    GEN::template coef<MMAX>(gp + sys * (kp.M_gen - 1) * 3, kp.M_gen, mid_t + c_mid * dt, g1);
-                    for (int m = 0; m < MMAX; ++m) sc[m] = g0[m], sc[MMAX + m] = g1[m];
-                }
+            const double t = ca.t[sys], h = ca.h[sys];
+            const int evk = exp_event_kind(kp, word, t, h, dt);
+            if (evk == VO_EV_STEP) {
+                const double c_mid = 0.288675134594812882254574390251;
+                const double mid_t = t + dt * 0.5;
+                double g0[MMAX], g1[MMAX];
+                GEN::template coef<MMAX>(gp + sys * (kp.M_gen - 1) * 3, kp.M_gen, mid_t - c_mid * dt, g0);
+                GEN::template coef<MMAX>(gp + sys * (kp.M_gen - 1) * 3, kp.M_gen, mid_t + c_mid * dt, g1);
+                for (int m = 0; m < MMAX; ++m) sc[m] = g0[m], sc[MMAX + m] = g1[m];
             }
-            si[0] = evk, sc[2 * MMAX] = dt;
+            si[0] = evk, si[1] = (evk == VO_EV_CHKPT || evk == VO_EV_END) ? (int)(word & VO_WORD_TGT_MASK) : -1, sc[2 * MMAX] = dt;
         }
         __syncthreads();
         int evk = si[0];
@@ -348,6 +338,8 @@ __global__ void __launch_bounds__(32 * NB) magnus_dense_kernel(const __grid_cons
                 }
                 __syncthreads();
             }
+        } else if (double2* dst = si[1] >= 0 ? exp_snap_row(kp, si[1], sys) : nullptr) {  // Chkpt / End: the state current() shows
+            for (int c = threadIdx.x; c < N; c += G::THREADS) dst[c] = psi[sys * N + c];
         }
         // ---- error norm, handle_step_adaptive (ode.rs:311-334), apply_step (ode.rs:402-428), masked commit
         if (evk == VO_EV_STEP && kp.adaptive) {

@@ -18,7 +18,14 @@ struct ExpKP {
     int nseq;             // mode 1: exponentials applied one after the other, coefficient sets [nseq][N][M]
     int n_events;         // mode 0, exp_small_kernel: events per system and launch (vo_exp_run fuses several; exp_step_kernel runs one)
     unsigned split_mask;  // VO_EXP_SPLIT_MIDPOINT: bit m set <=> basis matrix m belongs to split A
-    double t_end, t_start;
+    // ODEData.t_list (ode.rs:89): the first VO_INLINE_TLIST entries inline, a device copy of the whole list when it is longer
+    int n_tlist;
+    double t_list_inline[VO_INLINE_TLIST];
+    const double* t_list;
+    // nullable: [n_tlist][N][n], the state each system shows at its Chkpt / End event for t_list[k], row k of the CALLER's order:
+    // system `sys` of the device writes row snap_perm[sys] (vo_exp_set_order; NULL = the identity), so every snapshot is a plain view
+    double2* snap;
+    const int64_t* snap_perm;
     double rtol, alpha, pw, min_dt, max_dt;
     double norm1[VO_EXP_MAX_M];
     double cs[VO_EXP_MAX_M * VO_EXP_MAX_M * VO_EXP_MAX_M];
@@ -70,7 +77,8 @@ template <int NDIM, int M, int TB> struct Geo {
     static constexpr size_t SMEM_B = (size_t)M * 2 * NDIM * NDIM * sizeof(double);
     static constexpr size_t SMEM_T = (size_t)NBUF * 2 * TB * LDT * sizeof(double);
     static constexpr size_t SMEM_COEF = (size_t)VO_EXP_MAX_E * M * TB * sizeof(double2);
-    static constexpr size_t SMEM_MISC = (size_t)(NW * TB + VO_EXP_MAX_E * TB + TB) * sizeof(double) + (size_t)(TB + 2 * VO_EXP_MAX_E + 8) * sizeof(int) + (size_t)TB * sizeof(long long);
+    static constexpr size_t SMEM_MISC = (size_t)(NW * TB + VO_EXP_MAX_E * TB + TB) * sizeof(double) + (size_t)(TB + 2 * VO_EXP_MAX_E + 8) * sizeof(int) +
+                                        (size_t)TB * (sizeof(double2*) + sizeof(long long));
     static constexpr size_t SMEM = SMEM_B + SMEM_T + SMEM_COEF + SMEM_MISC;
     static_assert(SMEM <= 227 * 1024, "exp_step_kernel: shared memory budget of one SM exceeded");
 };
@@ -350,21 +358,28 @@ __device__ __forceinline__ void exp_counts_of(const ExpKP& kp, int* nbase, int* 
     *nerr = (kp.mode == 0 && kp.want_err) ? (tables ? kp.n_rows_err : (kp.scheme == VO_EXP_MAGNUS42 ? 1 : 0)) : 0;
 }
 
-// step_size_of (ode.rs:165-176) with t_list = [t0, tf]: the kind of this system's coming event (255: the trajectory is done) and,
-// for a step, its size dt.
+// step_size_of (ode.rs:165-176) + check_step (ode.rs:389-399) against t_list[tgt]: the kind of this system's coming event (255: the
+// trajectory is done) and, for a step, its size dt. Chkpt at every entry before the last, End at the last.
 __device__ __forceinline__ int exp_event_kind(const ExpKP& kp, uint32_t word, double t, double h, double& dt) {
     int evk = 255;
     if (!((word >> VO_WORD_STATUS_SHIFT) & VO_TRAJ_DONE)) {
         const int tgt = (int)(word & VO_WORD_TGT_MASK);
-        if (tgt >= 2) {
+        if (tgt >= kp.n_tlist) {
             evk = VO_EV_END;
         } else {
-            const double rem = (tgt == 0 ? kp.t_start : kp.t_end) - t;
-            if (fabs(rem) <= 2.220446049250313e-16) evk = tgt >= 1 ? VO_EV_END : VO_EV_CHKPT;
+            const double rem = (kp.n_tlist > VO_INLINE_TLIST ? kp.t_list[tgt] : kp.t_list_inline[tgt]) - t;
+            if (fabs(rem) <= 2.220446049250313e-16) evk = tgt >= kp.n_tlist - 1 ? VO_EV_END : VO_EV_CHKPT;
             else dt = rem < h ? rem : h, evk = VO_EV_STEP;
         }
     }
     return evk;
+}
+
+// Where system `sys` stores its state at its Chkpt / End event for t_list[tgt] (tgt: the target of the status word the event started
+// from), or NULL when snapshots are off or the target lies past the list. The caller stores row r of the state at [r].
+__device__ __forceinline__ double2* exp_snap_row(const ExpKP& kp, int tgt, int64_t sys) {
+    if (!kp.snap || tgt >= kp.n_tlist) return nullptr;
+    return kp.snap + ((int64_t)tgt * kp.N + (kp.snap_perm ? kp.snap_perm[sys] : sys)) * kp.n;
 }
 
 // The generator samples a step's exponents are built from (g: this system's generator parameters): midpoint at t + dt/2
@@ -551,6 +566,7 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
     int* sEv = reinterpret_cast<int*>(sDt + TB);                                                 // [TB] event, then [2 E] plan, [1] any
     int* sPlan = sEv + TB;
     long long* sSys = reinterpret_cast<long long*>(smem_raw + G::SMEM - TB * sizeof(long long));  // [TB] system of each tile slot (kp.N = none)
+    double2** sSnap = reinterpret_cast<double2**>(sSys - TB);  // [TB] snapshot row of the slot's Chkpt / End event of this tile, or NULL
     const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
     const int w = wi % G::NW, cg = wi / G::NW;
     const int row = 8 * w + (lane >> 2);
@@ -741,6 +757,7 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
                 const int s = threadIdx.x;
                 const int64_t sys = sSys[s];
                 int evk = sEv[s];
+                sSnap[s] = (evk == VO_EV_CHKPT || evk == VO_EV_END) ? exp_snap_row(kp, (int)(a_word & VO_WORD_TGT_MASK), sys) : nullptr;
                 if (evk != 255) {  // a_word, a_h: read in phase A by this thread; nothing has written them since
                     CtlAt c{ca, sys};
                     sEv[s] = exp_event_finish(kp, c, evk, a_word, a_h, sDt[s], [&]() {
@@ -767,6 +784,16 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
                     const int col = 16 * cg + 8 * j + 2 * (lane & 3) + q;
                     const int64_t sys = sSys[col];
                     if (sys < kp.N && sEv[col] == VO_EV_STEP) dst[sys * NDIM + row] = make_double2(xfr[j][q], xfi[j][q]);
+                }
+        }
+        if (kp.mode == 0 && kp.snap) {  // the unchanged state of the systems at a Chkpt / End event, each lane its own rows
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+#pragma unroll
+                for (int q = 0; q < 2; ++q) {
+                    const int col = 16 * cg + 8 * j + 2 * (lane & 3) + q;
+                    double2* dst = sSnap[col];
+                    if (dst) dst[row] = psi[sSys[col] * NDIM + row];
                 }
         }
         __syncthreads();  // sEv / sCoef are rewritten by the next tile

@@ -278,6 +278,9 @@ exp_small_kernel(const __grid_constant__ ExpKP kp, const __grid_constant__ Small
                     err = sqrt(nn);
 #endif
                 }
+            } else if (double2* dst = exp_snap_row(kp, (int)(word & VO_WORD_TGT_MASK), sys)) {  // Chkpt / End: the state current() shows at this event
+#pragma unroll
+                for (int r = 0; r < N; ++r) dst[r] = make_double2(xr[r], xi[r]);
             }
             const int fin = exp_event_finish(kp, c, evk, word, h, dt, [&]() { return err; }, cnt);
             if (fin == VO_EV_STEP) {

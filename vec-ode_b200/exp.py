@@ -229,6 +229,31 @@ class _ExpSolver:
         check(lib().vo_exp_with_step_range(self._h, dt_min, dt_max), self.ctx._h)
         return self
 
+    def set_t_list(self, t_list):
+        """Output times (ODEData.t_list, ode.rs:89) in place of [t0, tf]: every system raises Chkpt at each entry before the last
+        and End at the last (vo_exp_set_t_list). Before the first step, or after reset()."""
+        tl = np.ascontiguousarray(t_list, dtype=np.float64).ravel()
+        check(lib().vo_exp_set_t_list(self._h, _np_ptr(tl), tl.size), self.ctx._h)
+        return self
+
+    def enable_snapshots(self):
+        """Keep every system's state at its Chkpt / End event for each entry of t_list (vo_exp_enable_snapshots)."""
+        check(lib().vo_exp_enable_snapshots(self._h), self.ctx._h)
+        return self
+
+    def snapshot(self, k: int, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """The states at t_list[k], [N][n] complex in the caller's order (vo_exp_snapshot)."""
+        psi = np.empty((self.N, self.n), dtype=np.complex128) if out is None else out
+        check(lib().vo_exp_snapshot(self._h, k, _np_ptr(psi.view(np.float64))), self.ctx._h)
+        return psi
+
+    def snapshot_ensemble(self, k: int):
+        """Snapshot k as a device-side Ensemble view (one row of 2 n N doubles, the caller's order), for `Group.gather_placed`."""
+        from .base import Ensemble, _TensorOwner
+        h = _vp()
+        check(lib().vo_exp_snapshot_device(self._h, k, C.byref(h)), self.ctx._h)
+        return Ensemble(self.ctx, 1, 2 * self.n * self.N, _handle=h, _owner=_TensorOwner(self))
+
     def step(self) -> ODEState:
         res = StepResult()
         check(lib().vo_exp_step(self._h, C.byref(res)), self.ctx._h)
