@@ -458,6 +458,22 @@ int32_t vo_exp_set_t_list(vo_expsolver s, const double* t_list, int32_t n);
 int32_t vo_exp_enable_snapshots(vo_expsolver s);
 int32_t vo_exp_snapshot(vo_expsolver s, int32_t k, double* psi_host /* [N][n] (re,im) */);
 int32_t vo_exp_snapshot_device(vo_expsolver s, int32_t k, vo_ens* out);
+/* Observables (no reference counterpart: ODEData keeps checkpoints and nothing else). K operators O_k, [K][n][n] complex row-major
+ * and shared by the ensemble like the basis, 1 <= K <= VO_EXP_MAX_OBS. At every Chkpt / End event for t_list[j] the kernels compute,
+ * from the state a snapshot would keep (whether or not snapshots are on),
+ *     e[j][i][k] = sum_r conj(psi_r) sum_c O_k[r][c] psi_c
+ * complex and not normalised by <psi|psi>, so non-Hermitian operators (sigma_-, |0><1|) work; for a Hermitian O_k the imaginary part
+ * is rounding. vo_exp_set_observables uploads the operators and allocates [len][N][K] complex, zeroed; vo_exp_set_t_list re-allocates
+ * it and vo_exp_reset keeps the contents until the next run overwrites them, as for the snapshots. K = 0 with ops NULL turns
+ * observables off and frees the storage; K < 0, K > VO_EXP_MAX_OBS or K > 0 with ops NULL return VO_ERR_BAD_ARG. Refused with
+ * VO_ERR_STATE once a step / run has begun, accepted again after vo_exp_reset. Both readers speak the caller's order and return
+ * VO_ERR_BAD_ARG for j outside the list and VO_ERR_STATE when observables are off. vo_exp_expectation copies [N][K] (re, im) to the
+ * host; vo_exp_expectation_device returns a non-owning device view of one row of 2 K N doubles (destroy it with vo_ens_destroy),
+ * what vo_group_gather_placed takes. */
+#define VO_EXP_MAX_OBS 8
+int32_t vo_exp_set_observables(vo_expsolver s, int32_t K, const double* ops /* [K][n][n] (re,im) row-major */);
+int32_t vo_exp_expectation(vo_expsolver s, int32_t j, double* host /* [N][K] (re,im) */);
+int32_t vo_exp_expectation_device(vo_expsolver s, int32_t j, vo_ens* out);
 
 /* ---- multi-GPU: one ensemble sharded by trajectory over the GPUs of one box ------------------------------------------ */
 /* The reference has no parallelism of any kind; what replaces "one solver object per trajectory, run them in any order" is

@@ -187,6 +187,9 @@ SIGNATURES = {
     "vo_exp_enable_snapshots": (_i32, [_vp]),
     "vo_exp_snapshot": (_i32, [_vp, _i32, _vp]),
     "vo_exp_snapshot_device": (_i32, [_vp, _i32, _pvp]),
+    "vo_exp_set_observables": (_i32, [_vp, _i32, _vp]),
+    "vo_exp_expectation": (_i32, [_vp, _i32, _vp]),
+    "vo_exp_expectation_device": (_i32, [_vp, _i32, _pvp]),
     "vo_group_unique_id": (_i32, [_vp]),
     "vo_group_create_rank": (_i32, [_vp, _vp, _i32, _i32, _pvp]),
     "vo_group_create_local": (_i32, [_pvp, _i32, _pvp]),

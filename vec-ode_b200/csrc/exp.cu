@@ -73,6 +73,9 @@ struct vo_expsolver_s {
     std::vector<double> t_list;   // ODEData.t_list (ode.rs:89): [t0, tf] (ode.rs:144) unless vo_exp_set_t_list
     double* t_list_dev = nullptr;  // device copy of a list longer than VO_INLINE_TLIST
     double2* snap = nullptr;       // [t_list.size()][N][n] in the caller's order (vo_exp_enable_snapshots), else NULL
+    int n_obs = 0;                 // vo_exp_set_observables: K operators, 0 = off
+    double2* obs = nullptr;        // [n_obs][n][n] row-major
+    double2* obs_out = nullptr;    // [t_list.size()][N][n_obs] expectation values in the caller's order
     bool stepped = false;          // an event has run since creation or the last vo_exp_reset: the list is fixed until the next reset
     bool want_err = true;  // alph_err / x_err present (exp/cfm.rs:157-161)
     unsigned split_mask = 1u;  // VO_EXP_SPLIT_MIDPOINT: which basis matrices form split A (default: B_0)
@@ -353,7 +356,8 @@ int32_t exp_launch_event(vo_expsolver_s* s, bool adaptive, int events = 1) {
     kp.N = s->N, kp.count_events = 1, kp.n_events = events;
     kp.n_tlist = (int)s->t_list.size(), kp.t_list = s->t_list_dev;
     for (int i = 0; i < VO_INLINE_TLIST && i < kp.n_tlist; ++i) kp.t_list_inline[i] = s->t_list[i];
-    kp.snap = s->snap, kp.snap_perm = s->perm;
+    kp.snap = s->snap, kp.out_perm = s->perm;
+    kp.n_obs = s->n_obs, kp.obs = s->obs, kp.obs_out = s->obs_out;
     kp.rtol = s->rtol, kp.alpha = s->alpha, kp.pw = s->pw, kp.min_dt = s->min_dt, kp.max_dt = s->max_dt;
     kp.pw_is_third = s->pw == 1.0 / 3.0;
     kp.literal_norm = (s->literal_norm && adaptive) ? 1 : 0;
@@ -561,19 +565,20 @@ int32_t vo_exp_destroy(vo_expsolver s) {
     vo_dfree(s->ev_dev), cudaFreeHost(s->ev_host);
     rtc_exp_unload(s->gen_module);
     vo_dfree(s->perm), vo_dfree(s->stage);
-    vo_dfree(s->t_list_dev), vo_dfree(s->snap);
+    vo_dfree(s->t_list_dev), vo_dfree(s->snap), vo_dfree(s->obs), vo_dfree(s->obs_out);
     delete s;
     return VO_OK;
 }
 
-// Snapshot storage for the current list, zeroed: a system writes its row of entry k at its Chkpt / End event for t_list[k]
-static int32_t exp_alloc_snapshots(vo_expsolver_s* s) {
+// Output storage [len(t_list)][N][width] for the current list, zeroed: a system writes its row of entry k at its Chkpt / End event for
+// t_list[k] (snapshots: width n; expectation values: width n_obs)
+static int32_t exp_alloc_rows(vo_expsolver_s* s, double2** buf, int width) {
     vo_ctx c = s->ctx;
     VO_CUDA(c, cudaStreamSynchronize(c->stream));
-    vo_dfree(s->snap), s->snap = nullptr;
-    const size_t bytes = sizeof(double2) * s->t_list.size() * (size_t)s->N * s->sp->n;
-    if (vo_dmalloc(&s->snap, bytes) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "vo_exp_enable_snapshots: cudaMalloc failed");
-    VO_CUDA(c, cudaMemsetAsync(s->snap, 0, bytes, c->stream));
+    vo_dfree(*buf), *buf = nullptr;
+    const size_t bytes = sizeof(double2) * s->t_list.size() * (size_t)s->N * width;
+    if (vo_dmalloc(buf, bytes) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "exp: output storage: cudaMalloc failed");
+    VO_CUDA(c, cudaMemsetAsync(*buf, 0, bytes, c->stream));
     return VO_OK;
 }
 
@@ -857,14 +862,15 @@ int32_t vo_exp_set_t_list(vo_expsolver s, const double* t_list, int32_t n) {
         VO_CUDA(c, cudaMemcpy(s->t_list_dev, t_list, sizeof(double) * n, cudaMemcpyHostToDevice));
     }
     s->t_list.assign(t_list, t_list + n);
-    return s->snap ? exp_alloc_snapshots(s) : VO_OK;
+    int32_t r = s->snap ? exp_alloc_rows(s, &s->snap, s->sp->n) : VO_OK;
+    return r == VO_OK && s->n_obs ? exp_alloc_rows(s, &s->obs_out, s->n_obs) : r;
 }
 
 int32_t vo_exp_enable_snapshots(vo_expsolver s) {
     if (!s) return VO_ERR_BAD_ARG;
     if (s->snap) return VO_OK;
     DeviceGuard g(s->ctx->device);
-    return exp_alloc_snapshots(s);
+    return exp_alloc_rows(s, &s->snap, s->sp->n);
 }
 
 static int32_t exp_snapshot_check(vo_expsolver s, int32_t k) {
@@ -891,6 +897,52 @@ int32_t vo_exp_snapshot_device(vo_expsolver s, int32_t k, vo_ens* out) {
     if (r != VO_OK) return r;
     const int64_t row = (int64_t)s->N * s->sp->n;
     return vo_ens_wrap(s->ctx, s->snap + (size_t)k * row, 1, 2 * row, out);
+}
+
+int32_t vo_exp_set_observables(vo_expsolver s, int32_t K, const double* ops) {
+    if (!s || K < 0 || K > VO_EXP_MAX_OBS || (K > 0 && !ops)) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_set_observables: bad argument");
+    if (s->stepped) return vo_fail(s->ctx, VO_ERR_STATE, "vo_exp_set_observables: stepping has begun (vo_exp_reset rewinds it)");
+    vo_ctx c = s->ctx;
+    DeviceGuard g(c->device);
+    VO_CUDA(c, cudaStreamSynchronize(c->stream));
+    vo_dfree(s->obs), vo_dfree(s->obs_out), s->obs = nullptr, s->obs_out = nullptr, s->n_obs = 0;
+    if (K == 0) return VO_OK;
+    const size_t bytes = sizeof(double2) * (size_t)K * s->sp->n * s->sp->n;
+    if (vo_dmalloc(&s->obs, bytes) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "vo_exp_set_observables: cudaMalloc failed");
+    VO_CUDA(c, cudaMemcpy(s->obs, ops, bytes, cudaMemcpyHostToDevice));
+    int32_t r = exp_alloc_rows(s, &s->obs_out, K);
+    if (r != VO_OK) {
+        vo_dfree(s->obs), s->obs = nullptr;
+        return r;
+    }
+    s->n_obs = K;
+    return VO_OK;
+}
+
+static int32_t exp_expectation_check(vo_expsolver s, int32_t j) {
+    if (!s->n_obs) return vo_fail(s->ctx, VO_ERR_STATE, "vo_exp_expectation: observables are not set (vo_exp_set_observables)");
+    if (j < 0 || j >= (int32_t)s->t_list.size()) return vo_fail(s->ctx, VO_ERR_BAD_ARG, "vo_exp_expectation: index outside t_list");
+    return VO_OK;
+}
+
+int32_t vo_exp_expectation(vo_expsolver s, int32_t j, double* host) {
+    if (!s || !host) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_expectation: NULL argument");
+    int32_t r = exp_expectation_check(s, j);
+    if (r != VO_OK) return r;
+    vo_ctx c = s->ctx;
+    DeviceGuard g(c->device);
+    const size_t row = (size_t)s->N * s->n_obs;
+    VO_CUDA(c, cudaMemcpyAsync(host, s->obs_out + (size_t)j * row, sizeof(double2) * row, cudaMemcpyDeviceToHost, c->stream));
+    VO_CUDA(c, cudaStreamSynchronize(c->stream));
+    return VO_OK;
+}
+
+int32_t vo_exp_expectation_device(vo_expsolver s, int32_t j, vo_ens* out) {
+    if (!s || !out) return vo_fail(s ? s->ctx : nullptr, VO_ERR_BAD_ARG, "vo_exp_expectation_device: NULL argument");
+    int32_t r = exp_expectation_check(s, j);
+    if (r != VO_OK) return r;
+    const int64_t row = (int64_t)s->N * s->n_obs;
+    return vo_ens_wrap(s->ctx, s->obs_out + (size_t)j * row, 1, 2 * row, out);
 }
 
 

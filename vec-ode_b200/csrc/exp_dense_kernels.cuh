@@ -338,8 +338,11 @@ __global__ void __launch_bounds__(32 * NB) magnus_dense_kernel(const __grid_cons
                 }
                 __syncthreads();
             }
-        } else if (double2* dst = si[1] >= 0 ? exp_snap_row(kp, si[1], sys) : nullptr) {  // Chkpt / End: the state current() shows
-            for (int c = threadIdx.x; c < N; c += G::THREADS) dst[c] = psi[sys * N + c];
+        } else if (const int64_t orow = si[1] >= 0 ? exp_out_row(kp, si[1], sys) : -1; orow >= 0) {  // Chkpt / End: the state current() shows
+            if (kp.snap)
+                for (int c = threadIdx.x; c < N; c += G::THREADS) kp.snap[orow * N + c] = psi[sys * N + c];
+            if (kp.n_obs)  // one row in flight: more would push the kernel's step path into spills at n = 8 to 24
+                exp_expect_warp<1>(kp.obs, kp.n_obs, N, psi + sys * N, w, NB, kp.obs_out + orow * kp.n_obs);
         }
         // ---- error norm, handle_step_adaptive (ode.rs:311-334), apply_step (ode.rs:402-428), masked commit
         if (evk == VO_EV_STEP && kp.adaptive) {

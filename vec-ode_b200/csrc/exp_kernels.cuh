@@ -22,10 +22,15 @@ struct ExpKP {
     int n_tlist;
     double t_list_inline[VO_INLINE_TLIST];
     const double* t_list;
-    // nullable: [n_tlist][N][n], the state each system shows at its Chkpt / End event for t_list[k], row k of the CALLER's order:
-    // system `sys` of the device writes row snap_perm[sys] (vo_exp_set_order; NULL = the identity), so every snapshot is a plain view
+    // Output at every Chkpt / End event for t_list[k], row k of the CALLER's order: system `sys` of the device writes row
+    // out_perm[sys] (vo_exp_set_order; NULL = the identity), so every entry is a plain view (exp_out_row).
+    // snap (nullable): [n_tlist][N][n], the state the system shows at the event.
+    // obs_out (with n_obs > 0): [n_tlist][N][n_obs], <psi| O_k |psi> of that state for the operators obs [n_obs][n][n] (row-major).
     double2* snap;
-    const int64_t* snap_perm;
+    const int64_t* out_perm;
+    int n_obs;
+    const double2* obs;
+    double2* obs_out;
     double rtol, alpha, pw, min_dt, max_dt;
     double norm1[VO_EXP_MAX_M];
     double cs[VO_EXP_MAX_M * VO_EXP_MAX_M * VO_EXP_MAX_M];
@@ -78,7 +83,7 @@ template <int NDIM, int M, int TB> struct Geo {
     static constexpr size_t SMEM_T = (size_t)NBUF * 2 * TB * LDT * sizeof(double);
     static constexpr size_t SMEM_COEF = (size_t)VO_EXP_MAX_E * M * TB * sizeof(double2);
     static constexpr size_t SMEM_MISC = (size_t)(NW * TB + VO_EXP_MAX_E * TB + TB) * sizeof(double) + (size_t)(TB + 2 * VO_EXP_MAX_E + 8) * sizeof(int) +
-                                        (size_t)TB * (sizeof(double2*) + sizeof(long long));
+                                        (size_t)TB * 2 * sizeof(long long);
     static constexpr size_t SMEM = SMEM_B + SMEM_T + SMEM_COEF + SMEM_MISC;
     static_assert(SMEM <= 227 * 1024, "exp_step_kernel: shared memory budget of one SM exceeded");
 };
@@ -375,11 +380,45 @@ __device__ __forceinline__ int exp_event_kind(const ExpKP& kp, uint32_t word, do
     return evk;
 }
 
-// Where system `sys` stores its state at its Chkpt / End event for t_list[tgt] (tgt: the target of the status word the event started
-// from), or NULL when snapshots are off or the target lies past the list. The caller stores row r of the state at [r].
-__device__ __forceinline__ double2* exp_snap_row(const ExpKP& kp, int tgt, int64_t sys) {
-    if (!kp.snap || tgt >= kp.n_tlist) return nullptr;
-    return kp.snap + ((int64_t)tgt * kp.N + (kp.snap_perm ? kp.snap_perm[sys] : sys)) * kp.n;
+// The row of the [n_tlist][N] outputs that system `sys` writes at its Chkpt / End event for t_list[tgt] (tgt: the target of the status
+// word the event started from), or -1 when neither snapshots nor observables are on or the target lies past the list. The snapshot
+// goes to kp.snap + row n, the expectation values to kp.obs_out + row n_obs.
+__device__ __forceinline__ int64_t exp_out_row(const ExpKP& kp, int tgt, int64_t sys) {
+    if ((!kp.snap && !kp.n_obs) || tgt >= kp.n_tlist) return -1;
+    return (int64_t)tgt * kp.N + (kp.out_perm ? kp.out_perm[sys] : sys);
+}
+
+// dst[k] = <x| O_k |x> = sum_r conj(x_r) sum_c O_k[r][c] x_c for k = k0, k0 + dk, ... < n_obs (obs [n_obs][n][n]), by one warp (all 32
+// lanes call; n a multiple of 8, at most 64). Lane l owns columns c = l and l + 32: it forms (O_k^T conj(x))_c from coalesced reads of the operator
+// rows (ROWS of them in flight: the operators come from L2) and broadcast reads of x_r, multiplies by x_c, and a shuffle reduction
+// adds the lanes. x: one system's state in global memory, not written during the call.
+template <int ROWS>
+__device__ __forceinline__ void exp_expect_warp(const double2* __restrict__ obs, int n_obs, int n, const double2* x, int k0, int dk, double2* dst) {
+    const int lane = threadIdx.x & 31;
+    const double2 zero = make_double2(0.0, 0.0);
+    const double2 x0 = lane < n ? x[lane] : zero, x1 = lane + 32 < n ? x[lane + 32] : zero;
+    for (int k = k0; k < n_obs; k += dk) {
+        const double2* O = obs + (size_t)k * n * n;
+        double er = 0.0, ei = 0.0;
+#pragma unroll 1
+        for (int h = 0; h < 2 && 32 * h < n; ++h) {
+            const int c = lane + 32 * h;
+            const bool mine = c < n;
+            double ar = 0.0, ai = 0.0;
+#pragma unroll ROWS
+            for (int r = 0; r < n; ++r) {
+                const double2 o = mine ? O[r * n + c] : zero;
+                const double2 v = x[r];
+                ar = fma(v.x, o.x, fma(v.y, o.y, ar));
+                ai = fma(v.x, o.y, fma(-v.y, o.x, ai));
+            }
+            const double2 v = h ? x1 : x0;
+            er = fma(ar, v.x, fma(-ai, v.y, er));
+            ei = fma(ar, v.y, fma(ai, v.x, ei));
+        }
+        for (int o = 16; o > 0; o >>= 1) er += __shfl_xor_sync(0xffffffffu, er, o), ei += __shfl_xor_sync(0xffffffffu, ei, o);
+        if (lane == 0) dst[k] = make_double2(er, ei);
+    }
 }
 
 // The generator samples a step's exponents are built from (g: this system's generator parameters): midpoint at t + dt/2
@@ -566,7 +605,7 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
     int* sEv = reinterpret_cast<int*>(sDt + TB);                                                 // [TB] event, then [2 E] plan, [1] any
     int* sPlan = sEv + TB;
     long long* sSys = reinterpret_cast<long long*>(smem_raw + G::SMEM - TB * sizeof(long long));  // [TB] system of each tile slot (kp.N = none)
-    double2** sSnap = reinterpret_cast<double2**>(sSys - TB);  // [TB] snapshot row of the slot's Chkpt / End event of this tile, or NULL
+    long long* sRow = sSys - TB;  // [TB] output row (exp_out_row) of the slot's Chkpt / End event of this tile, or -1
     const int lane = threadIdx.x & 31, wi = threadIdx.x >> 5;
     const int w = wi % G::NW, cg = wi / G::NW;
     const int row = 8 * w + (lane >> 2);
@@ -757,7 +796,7 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
                 const int s = threadIdx.x;
                 const int64_t sys = sSys[s];
                 int evk = sEv[s];
-                sSnap[s] = (evk == VO_EV_CHKPT || evk == VO_EV_END) ? exp_snap_row(kp, (int)(a_word & VO_WORD_TGT_MASK), sys) : nullptr;
+                sRow[s] = (evk == VO_EV_CHKPT || evk == VO_EV_END) ? exp_out_row(kp, (int)(a_word & VO_WORD_TGT_MASK), sys) : -1;
                 if (evk != 255) {  // a_word, a_h: read in phase A by this thread; nothing has written them since
                     CtlAt c{ca, sys};
                     sEv[s] = exp_event_finish(kp, c, evk, a_word, a_h, sDt[s], [&]() {
@@ -792,10 +831,12 @@ exp_step_kernel(const __grid_constant__ ExpKP kp, const double* __restrict__ fra
 #pragma unroll
                 for (int q = 0; q < 2; ++q) {
                     const int col = 16 * cg + 8 * j + 2 * (lane & 3) + q;
-                    double2* dst = sSnap[col];
-                    if (dst) dst[row] = psi[sSys[col] * NDIM + row];
+                    if (sRow[col] >= 0) kp.snap[sRow[col] * NDIM + row] = psi[sSys[col] * NDIM + row];
                 }
         }
+        if (kp.mode == 0 && kp.n_obs)  // expectation values of the same unchanged states, one warp per slot
+            for (int s = wi; s < TB; s += G::THREADS / 32)
+                if (sRow[s] >= 0) exp_expect_warp<8>(kp.obs, kp.n_obs, NDIM, psi + sSys[s] * NDIM, 0, 1, kp.obs_out + sRow[s] * kp.n_obs);
         __syncthreads();  // sEv / sCoef are rewritten by the next tile
     }
     if (kp.mode == 0 && kp.count_events && threadIdx.x < 32) exp_counts_flush(ev + (blockIdx.x % VO_EV_SLOTS), cnt);

@@ -143,6 +143,33 @@ __device__ __forceinline__ void small_map_exp(const ExpKP& kp, const SmallBasis<
     }
 }
 
+// out[k] = <x| O_k |x> = sum_r conj(x_r) sum_c O_k[r][c] x_c for the n_obs operators obs [n_obs][N][N], from this thread's copy of the
+// state in shared memory (row r at xs[r * VO_EXP_SMALL_THREADS]). Every thread reads the operators at the same address, so each
+// load is a broadcast. Called at Chkpt / End events only, and not inlined: its code and registers stay out of the kernel's step
+// loop (DESIGN.md §2.3). Plain pointers rather than the launch parameters, which a call could only take by a local copy.
+template <int N>
+__device__ __noinline__ void small_expect(const double2* __restrict__ obs, int n_obs, const double2* xs, double2* out) {
+#pragma unroll 1
+    for (int k = 0; k < n_obs; ++k) {
+        double er = 0.0, ei = 0.0;
+#pragma unroll (N <= 4 ? N : 1)
+        for (int r = 0; r < N; ++r) {
+            const double2* O = obs + (k * N + r) * N;
+            double ar = 0.0, ai = 0.0;
+#pragma unroll
+            for (int c = 0; c < N; ++c) {
+                const double2 o = O[c], x = xs[c * VO_EXP_SMALL_THREADS];
+                ar = fma(o.x, x.x, fma(-o.y, x.y, ar));
+                ai = fma(o.x, x.y, fma(o.y, x.x, ai));
+            }
+            const double2 v = xs[r * VO_EXP_SMALL_THREADS];
+            er = fma(v.x, ar, fma(v.y, ai, er));
+            ei = fma(v.x, ai, fma(-v.y, ar, ei));
+        }
+        out[k] = make_double2(er, ei);
+    }
+}
+
 // x <- exp(Omega) x for magnus_42 with the applied commutator, Omega = W1 + b2 [L0, L1] (w1, l0, l1: real coefficients). Up to n = 3
 // Omega is assembled once per exponential from the three operators (6 n^2 doubles at once); above, a Taylor term is
 // W1 T + b2 (L0 (L1 T) - L1 (L0 T)) by products, as exp_step_kernel's map_exp_tile_comm does.
@@ -278,9 +305,15 @@ exp_small_kernel(const __grid_constant__ ExpKP kp, const __grid_constant__ Small
                     err = sqrt(nn);
 #endif
                 }
-            } else if (double2* dst = exp_snap_row(kp, (int)(word & VO_WORD_TGT_MASK), sys)) {  // Chkpt / End: the state current() shows at this event
+            } else if (const int64_t row = exp_out_row(kp, (int)(word & VO_WORD_TGT_MASK), sys); row >= 0) {  // Chkpt / End: the state current() shows
+                if (kp.snap)
 #pragma unroll
-                for (int r = 0; r < N; ++r) dst[r] = make_double2(xr[r], xi[r]);
+                    for (int r = 0; r < N; ++r) kp.snap[row * N + r] = make_double2(xr[r], xi[r]);
+                if (kp.n_obs) {  // from x0's slot, free outside a step
+#pragma unroll
+                    for (int r = 0; r < N; ++r) sx0[r * VO_EXP_SMALL_THREADS + threadIdx.x] = make_double2(xr[r], xi[r]);
+                    small_expect<N>(kp.obs, kp.n_obs, sx0 + threadIdx.x, kp.obs_out + row * kp.n_obs);
+                }
             }
             const int fin = exp_event_finish(kp, c, evk, word, h, dt, [&]() { return err; }, cnt);
             if (fin == VO_EV_STEP) {

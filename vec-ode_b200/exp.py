@@ -164,6 +164,13 @@ def with_commutator_slot(B0: np.ndarray, B1: np.ndarray):
     return np.stack([B0, B1, comm]), cs
 
 
+def _checked_out(out, shape, what):
+    """A caller's output buffer that the C ABI fills with shape[0] * shape[1] complex numbers: exactly that, contiguous."""
+    if not isinstance(out, np.ndarray) or out.dtype != np.complex128 or out.shape != shape or not out.flags.c_contiguous:
+        raise _cabi.VecOdeError(_cabi.VO_ERR_SHAPE, f"{what}: `out` must be a C-contiguous complex128 array of shape {shape}")
+    return out
+
+
 class _ExpSolver:
     SCHEME = None
 
@@ -178,6 +185,7 @@ class _ExpSolver:
         self.M_gen = sp.M if M_gen is None else M_gen
         gp = np.ascontiguousarray(gp, dtype=np.float64).reshape(self.N, max(self.M_gen - 1, 0), 3)
         self._perm = None
+        self._n_obs = 0  # operators of set_observables
         if group_similar and self.M_gen > 1:
             key = (np.abs(gp[:, :, 0]) * sp.norm1[1:self.M_gen][None, :]).sum(axis=1)
             self._perm = np.ascontiguousarray(np.argsort(key, kind="stable"), dtype=np.int64)
@@ -243,7 +251,7 @@ class _ExpSolver:
 
     def snapshot(self, k: int, out: Optional[np.ndarray] = None) -> np.ndarray:
         """The states at t_list[k], [N][n] complex in the caller's order (vo_exp_snapshot)."""
-        psi = np.empty((self.N, self.n), dtype=np.complex128) if out is None else out
+        psi = np.empty((self.N, self.n), dtype=np.complex128) if out is None else _checked_out(out, (self.N, self.n), "snapshot")
         check(lib().vo_exp_snapshot(self._h, k, _np_ptr(psi.view(np.float64))), self.ctx._h)
         return psi
 
@@ -253,6 +261,37 @@ class _ExpSolver:
         h = _vp()
         check(lib().vo_exp_snapshot_device(self._h, k, C.byref(h)), self.ctx._h)
         return Ensemble(self.ctx, 1, 2 * self.n * self.N, _handle=h, _owner=_TensorOwner(self))
+
+    def set_observables(self, ops):
+        """Expectation values <psi| O_k |psi> (complex, not normalised) of every system at each entry of t_list, computed in the
+        kernels at the Chkpt / End event (vo_exp_set_observables). `ops`: one n x n matrix or [K][n][n], 1 <= K <= 8, shared by the
+        ensemble; None turns them off. Before the first step, or after reset()."""
+        if ops is None:
+            check(lib().vo_exp_set_observables(self._h, 0, None), self.ctx._h)
+            self._n_obs = 0
+            return self
+        a = np.asarray(ops, dtype=np.complex128)
+        if a.ndim == 2:
+            a = a[None]
+        if a.ndim != 3 or a.shape[1:] != (self.n, self.n):
+            raise _cabi.VecOdeError(_cabi.VO_ERR_SHAPE, f"set_observables: operators must be [K][{self.n}][{self.n}], got {a.shape}")
+        a = np.ascontiguousarray(a)
+        check(lib().vo_exp_set_observables(self._h, a.shape[0], _np_ptr(a.view(np.float64))), self.ctx._h)
+        self._n_obs = a.shape[0]
+        return self
+
+    def expectation(self, j: int, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """<psi| O_k |psi> at t_list[j], [N][K] complex in the caller's order (vo_exp_expectation)."""
+        e = np.empty((self.N, max(self._n_obs, 1)), dtype=np.complex128) if out is None else _checked_out(out, (self.N, self._n_obs), "expectation")
+        check(lib().vo_exp_expectation(self._h, j, _np_ptr(e.view(np.float64))), self.ctx._h)
+        return e
+
+    def expectation_ensemble(self, j: int):
+        """Expectation values at t_list[j] as a device-side Ensemble view (one row of 2 K N doubles, the caller's order)."""
+        from .base import Ensemble, _TensorOwner
+        h = _vp()
+        check(lib().vo_exp_expectation_device(self._h, j, C.byref(h)), self.ctx._h)
+        return Ensemble(self.ctx, 1, 2 * self._n_obs * self.N, _handle=h, _owner=_TensorOwner(self))
 
     def step(self) -> ODEState:
         res = StepResult()
