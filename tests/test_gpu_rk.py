@@ -267,26 +267,6 @@ def test_heat_ensemble_kernel(vo, ctx, oracle):
         assert np.array_equal(got[i], rx)
 
 
-def test_t_list_checkpoints(vo, ctx, oracle):
-    """Multi-entry t_list (pub field ODEData.t_list, ode.rs:89): steps are clipped to land on each entry, a Chkpt is
-    emitted there and h is restored from prev_h (ode.rs:192-195) — lock-step and per-trajectory control."""
-    n = 64
-    kind, d, params, x0 = _case(vo, "HARMONIC2D", n, seed=5)
-    t_list = [0.0, 0.35, 0.5, 1.0]
-    otab = oracle.builtin_tableau(0)
-    for adaptive in (False, True):
-        ref = oracle.rk_ensemble(kind, params, otab, 0.0, 1.0, x0, 0.01, n_threads=2, adaptive=adaptive, rtol=1e-7, t_list=t_list)
-        rhs = _make_rhs(vo, ctx, kind, d, params)
-        s = vo.RK45Solver(rhs, 0.0, 1.0, vo.Ensemble.from_host(ctx, x0), 0.01).with_tolerance(1e-7, 1e-7).set_t_list(t_list)
-        st = s.run(adaptive=adaptive)
-        assert st.kind == "Done" and st.counts["Chkpt"] == 3 * n and st.counts["End"] == n
-        x = s.current()[1].to_host()
-        if adaptive:
-            np.testing.assert_allclose(x, ref["x"], atol=1e-6)
-        else:
-            assert np.array_equal(x, ref["x"])
-
-
 def test_per_trajectory_initial_step(vo, ctx, oracle):
     n = 128
     kind, d, params, x0 = _case(vo, "HARMONIC2D", n, seed=9)
@@ -474,29 +454,6 @@ def test_full_size_properties_heat(vo, ctx):
         R = 1.0 + z + z * z / 2.0 + z ** 3 / 6.0 + z ** 4 / 24.0
         expect += amp * (R ** steps) * np.sin(2.0 * np.pi * kmode * j / d)
     assert np.abs(u - expect).max() <= 1e-12
-
-
-@pytest.mark.parametrize("adaptive", [False, True])
-@pytest.mark.parametrize("stage_path", [False, True])
-def test_checkpoint_snapshots(vo, ctx, oracle, adaptive, stage_path):
-    """Checkpoint output (ODEData.t_list + Chkpt events, ode.rs:165-176, 192-195): the snapshot of entry k is the state
-    current() shows at that event = the final state of an oracle solve whose t_list stops at entry k."""
-    n = 96
-    kind, d, params, x0 = _case(vo, "HARMONIC2D", n, seed=11)
-    t_list = [0.0, 0.3, 0.55, 1.0]
-    rhs = _make_rhs(vo, ctx, kind, d, params)
-    s = vo.RK45Solver(rhs, 0.0, 1.0, vo.Ensemble.from_host(ctx, x0), 0.01).with_tolerance(1e-7, 1e-7).set_t_list(t_list)
-    s.set_stage_path(stage_path).enable_snapshots()
-    assert s.run(adaptive=adaptive).kind == "Done"
-    otab = oracle.builtin_tableau(0)
-    for k in range(len(t_list)):
-        ref = oracle.rk_ensemble(kind, params, otab, 0.0, t_list[k], x0, 0.01, n_threads=2, adaptive=adaptive, rtol=1e-7, t_list=t_list[:k + 1])
-        got = s.snapshot(k).to_host()
-        if adaptive:
-            np.testing.assert_allclose(got, ref["x"], atol=1e-6)
-        else:
-            assert np.array_equal(got, ref["x"]), k
-    assert np.array_equal(s.snapshot(len(t_list) - 1).to_host(), s.current()[1].to_host())
 
 
 @pytest.mark.parametrize("n", [4096, 512])  # two-trajectory kernel / one-trajectory staged kernel
@@ -775,13 +732,17 @@ def test_mixed_step_and_step_adaptive(vo, ctx, oracle):
     assert np.array_equal(s.stats()["h"], h_before_last)
 
 
-@pytest.mark.parametrize("n", [1024, 1026, 2500, 8192, 40_000, 65_538])
-def test_one_event_sweep_equals_stage_path_bitwise(vo, n):
+SWEEP_LISTS = {"": (0.0, 0.4, 1.0, 1.5), "-41": tuple(np.linspace(0.0, 1.5, 41))}  # 4 output times (inline) and 41 (device memory)
+
+
+@pytest.mark.parametrize("n,t_list", [pytest.param(n, tl, id=f"{n}{key}") for key, tl in SWEEP_LISTS.items()
+                                      for n in (1024, 1026, 2500, 8192, 40_000, 65_538)])
+def test_one_event_sweep_equals_stage_path_bitwise(vo, n, t_list):
     """The one-event adaptive sweep of the register-resident path (rk_small2.cuh: rk_ctl2w_staged_kernel, its slow path and
     ragged tail through ctl_lane) against the stage path in strict arithmetic (FAST's reformulated controller exists only on
     the register path): every bit of the state, of the controller arrays and of the snapshots must agree — through
     checkpoints, snapshots, ragged tails (n % 256 != 0), reads in mid-run, a write to the borrowed ensemble, a parameter
-    change and a switch to the 8-event kernel and back. The public state layout is the only one: set_blocked(False) is
+    change and a switch to the 8-event kernel and back; with 4 output times (inline) and 41 (read from device memory). The public state layout is the only one: set_blocked(False) is
     accepted, set_blocked(True) refused."""
     c = vo.Context(0, arith="strict")
     mu = vo.workloads.vdp_mu(n)
@@ -790,7 +751,7 @@ def test_one_event_sweep_equals_stage_path_bitwise(vo, n):
     for stage_path in (False, True):
         rhs = vo.Rhs(c, "VDP", 2, [mu])
         s = vo.RK45Solver(rhs, 0.0, 1.5, vo.Ensemble.from_host(c, x0), 1e-3, tableau=vo.ButcherTableu.builtin("DOPRI5")).with_tolerance(1e-6, 1e-6)
-        s.set_blocked(False).set_stage_path(stage_path).set_events_per_launch(1).set_t_list([0.0, 0.4, 1.0, 1.5]).enable_snapshots()
+        s.set_blocked(False).set_stage_path(stage_path).set_events_per_launch(1).set_t_list(t_list).enable_snapshots()
         with pytest.raises(vo.VecOdeError):
             s.set_blocked(True)
         for _ in range(25):
@@ -809,7 +770,7 @@ def test_one_event_sweep_equals_stage_path_bitwise(vo, n):
         s.set_events_per_launch(1)
         st = s.run(adaptive=True)                         # ... and back to the one-event sweep until every trajectory is done
         assert st.kind == "Done"
-        out.append((s.current()[1].to_host(), s.stats(), mid, [s.snapshot(k).to_host() for k in range(4)]))
+        out.append((s.current()[1].to_host(), s.stats(), mid, [s.snapshot(k).to_host() for k in range(len(t_list))]))
     (xa, sa, ma, snapa), (xb, sb, mb, snapb) = out
     assert np.array_equal(xa, xb)
     for k in ("accepted", "rejected", "t", "h", "dx_norm", "status"):

@@ -48,7 +48,8 @@ struct CtlShared {
     int pw_is_third;   // pw == 1.0/3.0 exactly (the order RK45Solver hard-wires, rk.rs:258-260)
     int record_dx_norm;  // keep ODEAdaptiveData.dx_norm (ode.rs:104) per trajectory
     int lazy_prev_h;     // two-trajectory control kernels: write prev_h only when its one reader (the Chkpt / End branch) comes next
-    double* snap;        // optional [n_tlist][d][N]: the state each trajectory shows at its Chkpt / End events, else NULL
+    double* snap;        // optional [n_tlist][snap_stride]: the state ([d][N]) each trajectory shows at its Chkpt / End events, else NULL
+    int64_t snap_stride; // d * N rounded up to even, so that every entry's block starts 16-byte aligned
 };
 
 // Event counters, VO_EV_SLOTS copies 128 bytes apart to spread the atomics (host sums the slots).
@@ -590,7 +591,7 @@ __device__ __forceinline__ void ctl_lane(const SoaAcc& a, const TableauDev& tb, 
         } else {  // Chkpt / End -> checkpoint_update, ode.rs:192-195
             if (cs.snap && tgt < cs.n_tlist) {  // what current() shows the caller at this event
 #pragma unroll
-                for (int c = 0; c < D; ++c) cs.snap[((int64_t)tgt * D + c) * a.count() + a.gidx()] = xc[c];
+                for (int c = 0; c < D; ++c) cs.snap[tgt * cs.snap_stride + (int64_t)c * a.count() + a.gidx()] = xc[c];
             }
             if (!prev_h_loaded) prev_h = a.ld_prev_h(), prev_h_loaded = true;
             tgt += 1, h = prev_h, ctl_dirty = true;

@@ -100,6 +100,8 @@ bool use_err(const vo_solver_s* s) { return s->tab.has_err && s->has_x_err; }
 // events per launch (the FP64 pipe, not HBM, then bounds a sweep).
 int step_fusion(const vo_solver_s* s) { return s->k_events > 0 ? s->k_events : 1; }
 int run_fusion(const vo_solver_s* s) { return s->k_events > 0 ? s->k_events : (s->uniform ? 16 : 8); }
+// Snapshot blocks: [d][N] per entry of t_list, each starting 16-byte aligned (vo_ens_wrap) even when d * N is odd.
+int64_t snap_stride(const vo_solver_s* s) { return (s->d * s->n + 1) & ~(int64_t)1; }
 
 TableauDev make_tableau_dev(const vo_tableau_s& t) {
     TableauDev d;
@@ -130,7 +132,7 @@ CtlShared make_ctl_shared(const vo_solver_s* s, int adaptive, int k_events) {
     cs.pw_is_third = s->pw == 1.0 / 3.0 ? 1 : 0;
     cs.record_dx_norm = s->record_dx_norm;
     cs.lazy_prev_h = s->mixed_stepping ? 0 : 1;
-    cs.snap = s->snap;
+    cs.snap = s->snap, cs.snap_stride = snap_stride(s);
     return cs;
 }
 
@@ -145,7 +147,7 @@ int uni_step_size(const vo_solver_s* s, double* dt) {
 void uni_checkpoint(vo_solver_s* s, bool end) {
     if (s->snap && s->u_tgt < (int)s->t_list.size()) {  // lock-step: the whole ensemble is at the checkpoint, copy it (stream-ordered)
         vo_touch(s->ctx);                                // the copy is not part of the CTA chain
-        cudaMemcpyAsync(s->snap + (size_t)s->u_tgt * s->d * s->n, s->x->p, sizeof(double) * s->d * s->n, cudaMemcpyDeviceToDevice, s->ctx->stream);
+        cudaMemcpyAsync(s->snap + (size_t)s->u_tgt * snap_stride(s), s->x->p, sizeof(double) * s->d * s->n, cudaMemcpyDeviceToDevice, s->ctx->stream);
     }
     s->u_tgt += 1, s->u_h = s->u_prev_h;
     if (end) s->u_done = true;
@@ -238,7 +240,7 @@ __global__ void ctl_commit_kernel(double* __restrict__ x, const double* __restri
             }
         } else {
             if (cs.snap && tgt < cs.n_tlist)
-                for (int64_t c = 0; c < d; ++c) cs.snap[((int64_t)tgt * d + c) * N + i] = x[c * N + i];
+                for (int64_t c = 0; c < d; ++c) cs.snap[tgt * cs.snap_stride + c * N + i] = x[c * N + i];
             tgt += 1, ca.h[i] = ca.prev_h[i];
             if (evk == VO_EV_END) status |= VO_TRAJ_DONE, ++c_end;
             else ++c_chkpt;
@@ -764,7 +766,7 @@ static int32_t alloc_snapshots(vo_solver s) {
     vo_ctx c = s->ctx;
     VO_CUDA(c, cudaStreamSynchronize(c->stream));
     vo_dfree(s->snap), s->snap = nullptr;
-    const size_t bytes = sizeof(double) * s->t_list.size() * (size_t)s->d * (size_t)s->n;
+    const size_t bytes = sizeof(double) * s->t_list.size() * (size_t)snap_stride(s);
     if (vo_dmalloc(&s->snap, bytes) != cudaSuccess) return vo_fail(c, VO_ERR_ALLOC, "vo_solver_enable_snapshots: cudaMalloc failed");
     VO_CUDA(c, cudaMemsetAsync(s->snap, 0, bytes, c->stream));
     return VO_OK;
@@ -1091,7 +1093,7 @@ int32_t vo_solver_snapshot(vo_solver s, int32_t k, vo_ens* out) {
     if (!s || !out) return VO_ERR_BAD_ARG;
     if (!s->snap) return vo_fail(s->ctx, VO_ERR_STATE, "vo_solver_snapshot: snapshots are not enabled");
     if (k < 0 || k >= (int32_t)s->t_list.size()) return vo_fail(s->ctx, VO_ERR_BAD_ARG, "vo_solver_snapshot: index outside t_list");
-    return vo_ens_wrap(s->ctx, s->snap + (size_t)k * s->d * s->n, s->d, s->n, out);
+    return vo_ens_wrap(s->ctx, s->snap + (size_t)k * snap_stride(s), s->d, s->n, out);
 }
 
 int32_t vo_step_many(const vo_solver* solvers, int32_t n, int32_t adaptive, int64_t rounds) {
