@@ -92,10 +92,12 @@ def exp_ensemble(scheme, basis, gp, psi0, t0, tf, h0, t_list=None, snapshots=Fal
 
 
 def solve(scheme, sp, gp_i, M_gen, psi0, t0, tf, h, t_list=None, adaptive=False, rtol=1e-4, min_dt=1e-6, max_dt=1.0, order=3.0,
-          alpha=0.9, max_calls=0, cs=None):
+          alpha=0.9, max_calls=0, cs=None, adaptive_from=None):
     """One system through ODEData / ODEAdaptiveData (base/ode.rs:79-206, 249-253, 311-341) as orc_exp_ensemble drives it:
     step_size_of against t_list[tgt_t] (ode.rs:165-176), the scheme's try_step (exp_oracle.py), the controller on the 2-norm of the
-    embedded error when `adaptive`, then advance / checkpoint_update. Returns dict(x, t, h, accepted, rejected, events, snap):
+    embedded error when `adaptive`, then advance / checkpoint_update. `adaptive_from` = c: calls 0 .. c-1 are step() (fixed), calls
+    from c on step_adaptive(), as a caller who switches in mid-list makes them (None: `adaptive` for every call).
+    Returns dict(x, t, h, accepted, rejected, events, dt, snap): `dt[j]` the step size of call j (0.0 for Chkpt / End),
     `snap[k]` the state x at the Chkpt / End event for t_list[k]."""
     from oracle.vecode_oracle import _libm, _rmax, _rmin, check_step
     g = eo.gen_cos(gp_i, M_gen, sp.M)
@@ -103,22 +105,23 @@ def solve(scheme, sp, gp_i, M_gen, psi0, t0, tf, h, t_list=None, adaptive=False,
     tl = [t0, tf] if t_list is None else list(t_list)
     x, t, tgt, cur_h, prev_h = list(psi0), t0, 0, h, h
     acc = rej = calls = 0
-    events, snap = [], [None] * len(tl)
+    events, dts, snap = [], [], [None] * len(tl)
     pw = 1.0 / order
     while max_calls <= 0 or calls < max_calls:
+        ada = adaptive if adaptive_from is None else calls >= adaptive_from
         calls += 1
         ev, dt = (END, 0.0) if tgt >= len(tl) else (STEP, check_step(t, tl[tgt], cur_h))
         if ev == STEP and dt is None:
-            ev = END if tgt >= len(tl) - 1 else CHKPT
+            ev, dt = (END if tgt >= len(tl) - 1 else CHKPT), 0.0
         h0 = cur_h
         if ev == STEP:
             if scheme == "midpoint":
                 xf, xe = eo.midpoint(sp, g, t, x, dt), None
             elif scheme == "cfm4":
-                xf, xe = eo.cfm_general(sp, gv, t, x, dt, eo.C_GAUSS_LEGENDRE_4, eo.CFM_R4_J2_GL, eo.CFM_R2_J1_GL if adaptive else None)
+                xf, xe = eo.cfm_general(sp, gv, t, x, dt, eo.C_GAUSS_LEGENDRE_4, eo.CFM_R4_J2_GL, eo.CFM_R2_J1_GL if ada else None)
             else:
-                xf, xe = eo.magnus_42(sp, g, t, x, dt, cs, want_err=adaptive)
-            if adaptive:  # handle_step_adaptive, ode.rs:311-334
+                xf, xe = eo.magnus_42(sp, g, t, x, dt, cs, want_err=ada)
+            if ada:  # handle_step_adaptive, ode.rs:311-334
                 nn = 0.0
                 for a, b in xe:
                     nn = nn + (a * a + b * b)
@@ -129,6 +132,7 @@ def solve(scheme, sp, gp_i, M_gen, psi0, t0, tf, h, t_list=None, adaptive=False,
                 if f <= 1.0:
                     ev = REJECT
         events.append(ev)
+        dts.append(dt)
         if ev == STEP:  # advance, ode.rs:184-188
             x, t = xf, t + dt
             acc += 1
@@ -140,4 +144,4 @@ def solve(scheme, sp, gp_i, M_gen, psi0, t0, tf, h, t_list=None, adaptive=False,
             tgt, cur_h = tgt + 1, prev_h
             if ev == END:
                 break
-    return dict(x=x, t=t, h=cur_h, accepted=acc, rejected=rej, events=events, snap=snap)
+    return dict(x=x, t=t, h=cur_h, accepted=acc, rejected=rej, events=events, dt=dts, snap=snap)

@@ -128,3 +128,98 @@ def test_checkpoint_kernels_compile_without_a_gpu(vo, n):
     """The kernels that read the list and write the snapshots, compiled at run time with a user generator and with a user norm."""
     assert vo.ExpCFMSolver.check_generator("g[1] = p[0] * cos(p[1] * t + p[2]);", n, 2) > 5_000
     assert vo.NormFn.check_kernels("m = e * e + im * im;", "sum", "r = sqrt(acc);", exp_n=n, exp_M=2) > 5_000
+
+
+# the edge lists of tests/test_gpu_exp_checkpoints.py, absolute times, h = 0.1: a first entry after t0, 0.2 twice, 4.2 / 4.25 / 4.3
+# closer together than h, and 3.0 -> 3.3 -> 4.2, 4.3 -> 4.5 in full steps whose sum falls one ulp short of the entry (a clipped
+# step of one ulp follows). EDGE8 (8 entries) is held inline in the launch parameters, EDGE (9) is read from device memory.
+EDGE8 = [0.2, 0.2, 3.0, 3.3, 4.2, 4.25, 4.3, 4.5]
+EDGE = [0.2, 0.2, 3.0, 3.3, 4.2, 4.2, 4.25, 4.3, 4.5]
+ONE = [1.0]
+EDGE_LISTS = {"EDGE8": EDGE8, "EDGE": EDGE, "ONE": ONE}
+# adaptive runs on the edge lists: the step capped at h = 0.1 so that slow systems walk the same grid; the solvers' initial step is then
+# sqrt(min_dt max_dt) (vo_exp_with_step_range, ode.rs:273-280)
+EDGE_RANGE = dict(min_dt=1e-6, max_dt=0.1)
+EDGE_H0 = float(np.sqrt(1e-6 * 0.1))
+
+
+def _with_zero_state(psi0):
+    """The ensemble plus one system that starts at psi = 0: its embedded error is exactly 0, so f = rtol / 0 = inf."""
+    return np.concatenate([psi0, np.zeros((1, psi0.shape[1]), complex)])
+
+
+@pytest.mark.parametrize("scheme,adaptive", CASES)
+@pytest.mark.parametrize("lst", list(EDGE_LISTS))
+def test_edge_lists_cpp_equals_pure_python_bitwise(oracle, scheme, adaptive, lst):
+    """EDGE8, EDGE and ONE with a zero-state system: both restatements give the same bits of states, snapshots, t, h, counts and
+    events. The zero-state system keeps exact zeros and, adaptive, takes the controller's largest growth at every step."""
+    basis, gp, psi0, cs, sp = _case(scheme)
+    psi0 = _with_zero_state(psi0)
+    gp = np.concatenate([gp, gp[:1]])
+    t_list = EDGE_LISTS[lst]
+    kw = dict(adaptive=True, no_adaptive=False, rtol=1e-7, **EDGE_RANGE) if adaptive else dict(no_adaptive=True)
+    h = EDGE_H0 if adaptive else 0.1
+    cap = 2000
+    ref = tl.exp_ensemble(scheme, basis, gp, psi0, 0.0, t_list[-1], h, M_gen=2, cs=cs, t_list=t_list, snapshots=True, events_cap=cap, **kw)
+    for i in range(psi0.shape[0]):
+        py = tl.solve(scheme, sp, [tuple(r) for r in gp[i]], 2, [(z.real, z.imag) for z in psi0[i]], 0.0, t_list[-1], h, t_list=t_list,
+                      adaptive=adaptive, rtol=1e-7, cs=None if cs is None else cs.tolist(), **(EDGE_RANGE if adaptive else {}))
+        assert np.array_equal(_c(py["x"]).view(np.float64), ref["psi"][i].view(np.float64)), i
+        assert (py["accepted"], py["rejected"]) == (ref["accepted"][i], ref["rejected"][i])
+        assert py["t"] == ref["t"][i] and py["h"] == ref["h"][i]
+        ev = ref["events"][i]
+        assert len(py["events"]) < cap and list(ev[:len(py["events"])]) == py["events"]
+        assert py["events"].count(CHKPT) == len(t_list) - 1 and py["events"].count(END) == 1 and py["events"][-1] == END
+        assert py["events"][0] == STEP  # the first entry lies after t0
+        for k in range(len(t_list)):
+            assert np.array_equal(_c(py["snap"][k]).view(np.float64), ref["snap"][k, i].view(np.float64)), (i, k)
+        assert abs(py["t"] - t_list[-1]) <= 2.0 ** -52
+    z = ref["snap"][:, -1]
+    assert np.all(z.view(np.float64) == 0.0) and np.all(ref["psi"][-1].view(np.float64) == 0.0)
+    if lst != "ONE":
+        assert np.array_equal(ref["snap"][0], ref["snap"][1])  # 0.2 twice: two Chkpt with no step between them
+    if adaptive:
+        assert ref["rejected"][-1] == 0 and ref["h"][-1] == 0.1  # f = inf: factor 2 at every step, up to max_dt
+
+
+def test_edge_list_takes_one_ulp_steps():
+    """On EDGE with fixed h = 0.1 the full steps to 3.0, 4.2 and 4.5 fall one ulp short: each of those entries is reached by a clipped step
+    of less than 1e-14, directly before its Chkpt / End. Without these the edge list would not test the clipped step it claims to."""
+    basis, gp, psi0, cs, sp = _case("cfm4")
+    py = tl.solve("cfm4", sp, [tuple(r) for r in gp[0]], 2, [(z.real, z.imag) for z in psi0[0]], 0.0, 4.5, 0.1, t_list=EDGE)
+    ev, dt = py["events"], py["dt"]
+    tiny = [j for j in range(len(ev)) if ev[j] == STEP and 0.0 < dt[j] < 1e-14]
+    assert len(tiny) >= 2, tiny
+    assert all(ev[j + 1] in (CHKPT, END) for j in tiny)
+    # the step before each is a full one
+    assert all(dt[j - 1] == 0.1 for j in tiny)
+
+
+@pytest.mark.parametrize("scheme", ["cfm4", "magnus42"])
+def test_switch_to_adaptive_in_mid_list(oracle, scheme):
+    """solve(adaptive_from=c): step() for the first c calls, step_adaptive() after. From call 0 it is the C++ adaptive run bit for bit,
+    never (a switch past the last call) the fixed run; a switch after entry 2 of a 9-entry list keeps the fixed run's bits up to entry 2,
+    then runs the controller (rejections, other step counts) to the end of the list."""
+    basis, gp, psi0, cs, sp = _case(scheme)
+    L9 = [0.0, 0.0611, 0.1937, 0.3, 0.4226, 0.55, 0.7123, 0.8377, 1.0]
+    cap = 400
+    ref = {a: tl.exp_ensemble(scheme, basis, gp, psi0, 0.0, 1.0, 0.1, M_gen=2, cs=cs, t_list=L9, snapshots=True, events_cap=cap,
+                              **(dict(adaptive=True, no_adaptive=False, rtol=1e-7) if a else dict(no_adaptive=False)))
+           for a in (False, True)}
+    csl = None if cs is None else cs.tolist()
+    for i in range(psi0.shape[0]):
+        args = (scheme, sp, [tuple(r) for r in gp[i]], 2, [(z.real, z.imag) for z in psi0[i]], 0.0, 1.0, 0.1)
+        fixed = tl.solve(*args, t_list=L9, rtol=1e-7, cs=csl)
+        for c, a in ((0, True), (len(fixed["events"]) + 1, False)):
+            py = tl.solve(*args, t_list=L9, rtol=1e-7, cs=csl, adaptive_from=c)
+            r = ref[a]
+            assert np.array_equal(_c(py["x"]).view(np.float64), r["psi"][i].view(np.float64)), (i, c)
+            assert (py["accepted"], py["rejected"], py["t"], py["h"]) == (r["accepted"][i], r["rejected"][i], r["t"][i], r["h"][i])
+            assert py["events"] == list(r["events"][i][:len(py["events"])])
+        c = [j for j, e in enumerate(fixed["events"]) if e == CHKPT][2] + 1  # the call after entry 2's Chkpt
+        py = tl.solve(*args, t_list=L9, rtol=1e-7, cs=csl, adaptive_from=c)
+        assert py["events"][:c] == fixed["events"][:c]
+        for k in range(3):
+            assert py["snap"][k] == fixed["snap"][k], (i, k)
+        assert py["events"].count(CHKPT) == len(L9) - 1 and py["events"][-1] == END
+        assert py["accepted"] != fixed["accepted"] and abs(py["t"] - 1.0) <= 2.0 ** -52
